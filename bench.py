@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--qubits 32] [--depth 100] [--precision f32] [--fuse 1]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[3], SURVEY.md 8(d) item 4): n-qubit brickwork of
 depth D -- layer l applies `add_q2_var_gate(i+1, i)` for i = l mod 2, l mod 2 + 2, ...
@@ -460,9 +461,20 @@ def roofline_block(prof, dev_ms, steps, precision, local_qubits, kinds, clocks, 
     return r
 
 
+def dump_outputs(out_dir, dens, grads):
+    """What a caller of the timed path receives from its last step, as real arrays with a trailing (real, imag) axis:
+    densities.npy (densities x 4 x 4 x 2) and gradients.npy (gates x gate entries x 2), float32 for f32 and float64
+    for f64.  The inputs are seeded, so two builds run with the same arguments can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, z in (("densities", np.stack([np.asarray(d) for d in dens])),
+                    ("gradients", np.stack([np.asarray(g).reshape(-1) for g in grads]))):
+        np.save(os.path.join(out_dir, name + ".npy"), np.stack([z.real, z.imag], axis=-1))
+
+
 def run_workload(args, world, rank, local, precision, workload, local_qubits, depth, warmup, steps, barrier,
-                 sample_clocks, check_sizes):
-    """Parity check, then the timed steps of one workload; returns the JSON fields (rank 0) or None."""
+                 sample_clocks, check_sizes, dump_dir=None):
+    """Parity check, then the timed steps of one workload; returns the JSON fields (rank 0) or None.  With dump_dir,
+    rank 0 also writes the outputs of the last timed step there (dump_outputs)."""
     import torch
     g = world.bit_length() - 1
     n_total = local_qubits + g
@@ -495,6 +507,8 @@ def run_workload(args, world, rank, local, precision, workload, local_qubits, de
     check = dict(check or {})
     check.update({"trace_density0": float(np.trace(dens[0]).real),
                   "grad_norm": float(np.sqrt(sum(np.vdot(x, x).real for x in grads)))})
+    if dump_dir:
+        dump_outputs(dump_dir, dens, grads)
     return {
         "metric": METRIC, "value": round(value, 3), "unit": UNIT, "n_gpus": world, "steps": steps,
         "warmup": warmup, "ms_per_step": round(dev_ms / steps, 3), "higher_is_better": True,
@@ -541,7 +555,7 @@ def run_ours(args):
 
     small = (24, 8) if args.workload == "brickwork" else (22, 3)
     out = run_workload(args, world, rank, local, args.precision, args.workload, args.qubits, args.depth, args.warmup,
-                       args.steps, barrier, True, small)
+                       args.steps, barrier, True, small, args.dump_outputs)
     # the other single-GPU BASELINE.json configs, each with its own roofline and parity check
     if world == 1 and args.secondary and args.workload == "brickwork" and args.precision == "f32" and args.qubits == 32:
         sec = {}
@@ -596,8 +610,8 @@ def run_reference(args):
         marks.append((name, ev))
 
     def step():
-        circ.forward([], var)
-        return circ.backward(cts_conj, [], var)
+        dens = circ.forward([], var)
+        return dens, circ.backward(cts_conj, [], var)
 
     for _ in range(args.warmup):
         step()
@@ -608,12 +622,14 @@ def run_reference(args):
     ev0.record()
     on_phase("start")
     for _ in range(args.steps):
-        step()
+        dens, grads = step()
     on_phase("end")
     ev1.record()
     torch.cuda.synchronize()
     wall = time.perf_counter() - t0
     dev_ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dens, grads)
     phase_ms = {"gates": 0.0, "densities": 0.0}
     for (name, a), (_, b) in zip(marks[:-1], marks[1:]):
         if name in phase_ms:
@@ -650,7 +666,9 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2)
+    ap.add_argument("--steps", type=int, default=2,
+                    help="timed steps of the workload; the secondary workloads (--secondary) run fixed counts: "
+                         "VQSE-28 5 steps, 32 q f64 1 step")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--qubits", type=int, default=32, help="LOCAL qubits per GPU (total = qubits + log2(gpus))")
@@ -675,7 +693,12 @@ def main():
     ap.add_argument("--no-check", action="store_true", help="skip the parity check that precedes the timed steps")
     ap.add_argument("--secondary", type=int, default=1,
                     help="1: after the default 32 q f32 run also measure VQSE-28 f32 and brickwork 32 q f64 (N = 1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the densities and gradients of the last timed step of the workload (not of the "
+                         "secondary workloads; with --impl reference, of its depth-bounded sample) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:
