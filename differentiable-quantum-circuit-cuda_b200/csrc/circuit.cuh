@@ -26,7 +26,8 @@
 enum Kind {
   K_CONST_Q2 = 0, K_VAR_Q2, K_CONST_Q2_NONU, K_VAR_Q2_NONU, K_CONST_Q2_DIAG, K_VAR_Q2_DIAG,
   K_CONST_Q1, K_CONST_Q1_NONU, K_VAR_Q1, K_VAR_Q1_NONU,
-  K_Q2_DENS, K_Q1_DENS, K_DIFF_Q2_DENS, K_DIFF_Q1_DENS
+  K_Q2_DENS, K_Q1_DENS, K_DIFF_Q2_DENS, K_DIFF_Q1_DENS,
+  K_DENS_K, K_DIFF_DENS_K   // densities on 3..6 qubits (add_dens; dens_k_kernels.cuh)
 };
 
 static inline bool kind_is_gate(int k) { return k <= K_VAR_Q1_NONU; }
@@ -40,7 +41,8 @@ static inline bool kind_is_diag(int k) { return k == K_CONST_Q2_DIAG || k == K_V
 static inline bool kind_is_q1(int k) { return k >= K_CONST_Q1 && k <= K_VAR_Q1_NONU; }
 static inline bool kind_is_q2dense(int k) { return k <= K_VAR_Q2_NONU; }
 static inline bool kind_is_dens(int k) { return k >= K_Q2_DENS; }
-static inline bool kind_is_diff_dens(int k) { return k == K_DIFF_Q2_DENS || k == K_DIFF_Q1_DENS; }
+static inline bool kind_is_diff_dens(int k) { return k == K_DIFF_Q2_DENS || k == K_DIFF_Q1_DENS || k == K_DIFF_DENS_K; }
+static inline bool kind_is_k_dens(int k) { return k == K_DENS_K || k == K_DIFF_DENS_K; }
 static inline bool kind_is_q1_dens(int k) { return k == K_Q1_DENS || k == K_DIFF_Q1_DENS; }
 static inline int kind_gate_len(int k) { return kind_is_q2dense(k) ? 16 : 4; }
 static inline int kind_dens_len(int k) { return kind_is_q1_dens(k) ? 4 : 16; }
@@ -48,7 +50,14 @@ static inline int kind_dens_len(int k) { return kind_is_q1_dens(k) ? 4 : 16; }
 struct Inst {
   int kind;
   int pos2, pos1;  // q1 kinds use pos2 only
+  int nk = 0;      // k-qubit densities: the qubits kpos[0..nk-1], most significant first (pos2 = pos1 = -1)
+  int kpos[6] = {-1, -1, -1, -1, -1, -1};
 };
+
+// complex entries of a density's output / cotangent
+static inline size_t dens_len(const Inst& in) {
+  return kind_is_k_dens(in.kind) ? (size_t)1 << (2 * in.nk) : (size_t)kind_dens_len(in.kind);
+}
 
 struct Stats {
   uint64_t kernel_launches = 0, hbm_passes = 0, algorithmic_bytes = 0;
@@ -56,6 +65,7 @@ struct Stats {
 
 struct DensGroup;
 struct TileDensParams;
+struct DensKParams;
 struct TcState;
 struct TcPass;
 
@@ -277,6 +287,16 @@ class Circuit {
   double* d_res_ = nullptr;  // device results: 32 doubles per slot
   size_t d_res_slots_ = 0;
   std::vector<double> h_res_;
+  // k-qubit densities: results (2 * 4^k doubles each, at kofs_[instruction]) and cotangents (4^k entries each,
+  // at kmat_ofs_[instruction]) in regions of their own
+  double* d_kres_ = nullptr;
+  size_t d_kres_cap_ = 0;
+  std::vector<double> h_kres_;
+  std::vector<size_t> kofs_;
+  cplx_t* d_kmat_ = nullptr;
+  size_t d_kmat_cap_ = 0;
+  std::vector<cplx_t> h_kmat_;
+  std::vector<size_t> kmat_ofs_;
   cudaStream_t stream_ = 0;
   Stats stats_;
   int opt_fuse_ = 2;          // 0: one pass per instruction, 1: tiled multi-gate passes, 2: + register-blocked forward
@@ -312,9 +332,14 @@ class Circuit {
     if (stage_a_) cudaFree(stage_a_);
     if (stage_b_) cudaFree(stage_b_);
     if (d_res_) cudaFree(d_res_);
+    if (d_kres_) cudaFree(d_kres_);
+    if (d_kmat_) cudaFree(d_kmat_);
     state_ = bwd_ = initial_ = stage_a_ = stage_b_ = nullptr;
     d_res_ = nullptr;
     d_res_slots_ = 0;
+    d_kres_ = nullptr;
+    d_kmat_ = nullptr;
+    d_kres_cap_ = d_kmat_cap_ = 0;
     ws_release(ws_);
     release_tiles();
 #ifndef QDC_F64
@@ -451,6 +476,7 @@ class Circuit {
   }
 
   const char* add(int kind, size_t pos2, size_t pos1) {
+    if (kind_is_k_dens(kind)) return qdc_errf("kind %d carries its qubits through qdc_circuit_add_dens.", kind);
     if (kind < 0 || kind > K_DIFF_Q1_DENS) return qdc_errf("Unknown instruction kind %d.", kind);
     const bool one = kind_is_q1(kind) || kind_is_q1_dens(kind);
     if (one) {
@@ -465,6 +491,25 @@ class Circuit {
     return nullptr;
   }
 
+  // Density on k = 1..6 qubits, positions[0] the most significant bit of its row and column index; k <= 2 adds the
+  // one- and two-qubit kinds.
+  const char* add_dens(const size_t* positions, size_t k, bool with_grad) {
+    if (k < 1 || k > 6) return qdc_errf("the number of density qubits must be in 1..6, got %zu.", k);
+    if (k == 1) return add(with_grad ? K_DIFF_Q1_DENS : K_Q1_DENS, positions[0], 0);
+    if (k == 2) return add(with_grad ? K_DIFF_Q2_DENS : K_Q2_DENS, positions[0], positions[1]);
+    Inst in{with_grad ? K_DIFF_DENS_K : K_DENS_K, -1, -1};
+    for (size_t j = 0; j < k; j++) {
+      if (positions[j] >= (size_t)n_) return qdc_errf("pos is out of the bound.");
+      for (size_t i = 0; i < j; i++)
+        if (positions[i] == positions[j]) return qdc_errf("positions must be different.");
+      in.kpos[j] = (int)positions[j];
+    }
+    in.nk = (int)k;
+    insts_.push_back(in);
+    forward_valid_ = false;
+    return nullptr;
+  }
+
   size_t count(int what) const {
     size_t c = 0;
     for (const Inst& in : insts_) {
@@ -475,8 +520,8 @@ class Circuit {
         case 2: c += kind_is_gate(k) && kind_is_var(k); break;
         case 3: c += kind_is_dens(k); break;
         case 4: c += kind_is_diff_dens(k); break;
-        case 5: c += kind_is_dens(k) ? kind_dens_len(k) : 0; break;
-        case 6: c += kind_is_diff_dens(k) ? kind_dens_len(k) : 0; break;
+        case 5: c += kind_is_dens(k) ? dens_len(in) : 0; break;
+        case 6: c += kind_is_diff_dens(k) ? dens_len(in) : 0; break;
         case 7: c += (kind_is_gate(k) && kind_is_var(k)) ? kind_gate_len(k) : 0; break;
       }
     }
@@ -652,6 +697,7 @@ class Circuit {
     if (kind_is_q1(k)) return 0;
     if (kind_is_q2dense(k)) return 1;
     if (kind_is_diag(k)) return 2;
+    if (kind_is_k_dens(k)) return 5;
     return kind_is_q1_dens(k) ? 3 : 4;
   }
 
@@ -726,6 +772,8 @@ class Circuit {
       si[i].q2 = insts_[i].pos2;
       si[i].q1 = insts_[i].pos1;
       si[i].skip = kind_is_dens(k) && !all_dens && !kind_is_diff_dens(k);
+      si[i].nq = insts_[i].nk;
+      for (int j = 0; j < insts_[i].nk; j++) si[i].qk[j] = insts_[i].kpos[j];
     }
     if (world_ > 1 && opt_auto_swap_pos_) {
       // sharded: where the remap victims may sit is decided by the cost model of scheduler.hpp (every rank builds the
@@ -984,8 +1032,27 @@ class Circuit {
     QDC_TRY(bind_gates(cg, vg, gp, false));
     const size_t need = count(all_dens ? 5 : 6);
     if (cap < need) return qdc_errf("Output buffer too small: %zu < %zu.", cap, need);
-    const size_t nslots = count(all_dens ? 3 : 4);
+    // 32-double slots of the one- and two-qubit densities; offsets of the k-qubit ones in their own region
+    size_t nslots = 0, nkres = 0;
+    kofs_.assign(insts_.size(), 0);
+    for (size_t i = 0; i < insts_.size(); i++) {
+      const Inst& in = insts_[i];
+      if (!kind_is_dens(in.kind) || (!all_dens && !kind_is_diff_dens(in.kind))) continue;
+      if (!kind_is_k_dens(in.kind)) {
+        nslots++;
+        continue;
+      }
+      kofs_[i] = nkres;
+      nkres += 2 * dens_len(in);
+    }
     QDC_TRY(ensure_results(nslots));
+    if (nkres > d_kres_cap_) {
+      if (d_kres_) QDC_CUDA(cudaFree(d_kres_));
+      d_kres_ = nullptr;
+      QDC_CUDA(cudaMalloc((void**)&d_kres_, nkres * sizeof(double)));
+      d_kres_cap_ = nkres;
+    }
+    h_kres_.resize(nkres);
     forward_valid_ = false;
     build_plan(all_dens);
     if (!plan_.ok)
@@ -1004,6 +1071,8 @@ class Circuit {
       QDC_CUDA(cudaMemcpyAsync(h_res_.data(), d_res_, nslots * 32 * sizeof(double), cudaMemcpyDeviceToHost,
                                stream_));
     }
+    if (nkres)
+      QDC_CUDA(cudaMemcpyAsync(h_kres_.data(), d_kres_, nkres * sizeof(double), cudaMemcpyDeviceToHost, stream_));
     QDC_CUDA(cudaStreamSynchronize(stream_));
     if (prof_.on) prof_.collect();
     size_t slot = 0, o = 0;
@@ -1011,6 +1080,16 @@ class Circuit {
       const Inst& in = insts_[i];
       if (!kind_is_dens(in.kind)) continue;
       if (!all_dens && !kind_is_diff_dens(in.kind)) continue;
+      if (kind_is_k_dens(in.kind)) {
+        const size_t len = dens_len(in);
+        const double* h = &h_kres_[kofs_[i]];
+        for (size_t j = 0; j < len; j++) {
+          out[o + j].x = (real_t)h[2 * j];
+          out[o + j].y = (real_t)h[2 * j + 1];
+        }
+        o += len;
+        continue;
+      }
       const double* h = &h_res_[slot * 32];
       if (kind_is_q1_dens(in.kind)) {
         for (int j = 0; j < 4; j++) {
@@ -1056,7 +1135,7 @@ class Circuit {
       long s = 0;
       for (size_t i = 0; i < insts_.size(); i++) {
         const int k = insts_[i].kind;
-        if (kind_is_dens(k) && (all_dens || kind_is_diff_dens(k))) dslot[i] = s++;
+        if (kind_is_dens(k) && !kind_is_k_dens(k) && (all_dens || kind_is_diff_dens(k))) dslot[i] = s++;
       }
     }
     const std::vector<qdc::Step>& steps = plan_.steps;
@@ -1142,7 +1221,7 @@ class Circuit {
         if (!kind_is_diff_dens(insts_[i].kind)) continue;
         if (di >= dg.count)
           return qdc_errf("The number of gradients wrt density matrices is less than required.");
-        if ((int)dg.lens[di] != kind_dens_len(insts_[i].kind))
+        if ((size_t)dg.lens[di] != dens_len(insts_[i]))
           return qdc_errf("Incorrect len of the gate's buffer.");
         dp[i] = dg.flat + off;
         off += dg.lens[di];
@@ -1150,12 +1229,30 @@ class Circuit {
       }
       if (di != dg.count) return qdc_errf("Number of gradients wrt density matrices is more than required.");
     }
+    // cotangents of the k-qubit densities go to the device in one copy (their seeds read them from there)
+    kmat_ofs_.assign(insts_.size(), 0);
+    h_kmat_.clear();
+    for (size_t i = 0; i < insts_.size(); i++) {
+      if (insts_[i].kind != K_DIFF_DENS_K) continue;
+      kmat_ofs_[i] = h_kmat_.size();
+      h_kmat_.insert(h_kmat_.end(), dp[i], dp[i] + dens_len(insts_[i]));
+    }
     const size_t need = count(7);
     if (cap < need) return qdc_errf("Output buffer too small: %zu < %zu.", cap, need);
     const size_t nvar = count(2);
     QDC_TRY(ensure_results(nvar));
     if (nvar) QDC_CUDA(cudaMemsetAsync(d_res_, 0, nvar * 32 * sizeof(double), stream_));
     if (!bwd_) QDC_CUDA(cudaMalloc((void**)&bwd_, bytes()));  // (sharded mode allocated it in shard())
+    if (!h_kmat_.empty()) {
+      if (h_kmat_.size() > d_kmat_cap_) {
+        if (d_kmat_) QDC_CUDA(cudaFree(d_kmat_));
+        d_kmat_ = nullptr;
+        QDC_CUDA(cudaMalloc((void**)&d_kmat_, h_kmat_.size() * sizeof(cplx_t)));
+        d_kmat_cap_ = h_kmat_.size();
+      }
+      QDC_CUDA(cudaMemcpyAsync(d_kmat_, h_kmat_.data(), h_kmat_.size() * sizeof(cplx_t), cudaMemcpyHostToDevice,
+                               stream_));
+    }
 
     // variable-gate slot of every instruction
     std::vector<long> vslot(insts_.size(), -1);
@@ -1366,6 +1463,12 @@ class Circuit {
   const char* run_seed_group(const DensGroup& g, const std::vector<const cplx_t*>& dp, bool live);
   const char* run_dens_run(size_t first, size_t last, const std::vector<long>& dslot);
   const char* run_seed_run(size_t first, size_t last, const std::vector<const cplx_t*>& dp, bool* live);
+  // k-qubit densities / seeds (dens_k_kernels.cuh)
+  const char* fill_dens_k_params(const qdc::Step& st, DensKParams* p);
+  template <int KQ> const char* launch_dens_k(const DensKParams& p, double* dst);
+  template <int KQ> const char* launch_seed_k(const DensKParams& p, const cplx_t* G);
+  const char* dens_k(const qdc::Step& st);
+  const char* seed_k(const qdc::Step& st, bool live);
   std::vector<char> diag_hilo_;  // diagonal gradient of this instruction came back in (hi,lo) order
   double* tile_partials_ = nullptr;
   size_t tile_partials_cap_ = 0;

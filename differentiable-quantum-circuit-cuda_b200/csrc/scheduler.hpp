@@ -10,7 +10,8 @@
 //    may be re-ordered within the dependency DAG defined by shared qubits.
 //  * Density instructions are full barriers (a Diff density must see exactly
 //    the gates that precede it in program order, otherwise the gradients of
-//    non-unitary directions change).
+//    non-unitary directions change).  A k-qubit density (kind class 5) needs
+//    all its k qubits local at once.
 //
 // Sharding: with 2^g ranks the top g PHYSICAL bit positions are the rank
 // index ("global").  A logical->physical qubit map is maintained; dense gates
@@ -41,6 +42,7 @@ struct Step {
   int first = 0, count = 0;  // TILE: range in Plan::tile_steps
   int tb_first = 0, tb_count = 0;  // TILE: range in Plan::tile_bits (sorted physical positions)
   int grp_first = 0, grp_count = 0;  // TILE: range in Plan::groups (register-block groups)
+  int nk = 0, pk[6] = {-1, -1, -1, -1, -1, -1};  // k-qubit DENS (p2 = p1 = -1): physical positions, most significant first
 };
 
 // A register-block group inside a tile pass: `count` consecutive tile gates
@@ -61,9 +63,11 @@ struct Plan {
 };
 
 struct SchedInst {
-  int kind_class;  // 0: dense q1, 1: dense q2, 2: diagonal q2, 3: density q1, 4: density q2
-  int q2, q1;      // logical qubits (q1 = -1 for one-qubit instructions)
+  int kind_class;  // 0: dense q1, 1: dense q2, 2: diagonal q2, 3: density q1, 4: density q2, 5: density on nq qubits
+  int q2, q1;      // logical qubits (q1 = -1 for one-qubit instructions; both -1 for class 5)
   bool skip;       // densities that this sweep does not evaluate
+  int nq = 0;      // class 5: the logical qubits qk[0..nq-1], most significant first
+  int qk[6] = {-1, -1, -1, -1, -1, -1};
 };
 
 struct SchedOptions {
@@ -141,7 +145,8 @@ class Scheduler {
       if (is_dens(s)) {
         // barrier: runs only if everything before it is done
         if (any_blocked) break;
-        const bool ok = local(s.q2) && (s.q1 < 0 || local(s.q1));
+        bool ok = s.nq > 0 || (local(s.q2) && (s.q1 < 0 || local(s.q1)));
+        for (int j = 0; j < s.nq; j++) ok = ok && local(s.qk[j]);
         if (!ok) break;
         ready.push_back(make_step(i, ST_DENS));
         done_[i] = true;
@@ -164,6 +169,11 @@ class Scheduler {
     Step st;
     st.type = type;
     st.inst = i;
+    if (in_[i].nq > 0) {
+      st.nk = in_[i].nq;
+      for (int j = 0; j < st.nk; j++) st.pk[j] = map_[in_[i].qk[j]];
+      return st;
+    }
     st.p2 = map_[in_[i].q2];
     st.p1 = in_[i].q1 >= 0 ? map_[in_[i].q1] : -1;
     return st;
@@ -443,6 +453,10 @@ class Scheduler {
     std::vector<int> nu(o_.n, N + 1);
     for (int i = N - 1; i >= 0; i--) {
       if (done_[i]) continue;
+      // (the qubits of a k-qubit density share one next use: a remap for it never evicts another of them, the
+      // victims must be strictly less urgent)
+      for (int j = 0; j < in_[i].nq; j++) nu[in_[i].qk[j]] = i;
+      if (in_[i].nq > 0) continue;
       nu[in_[i].q2] = i;
       if (in_[i].q1 >= 0) nu[in_[i].q1] = i;
     }

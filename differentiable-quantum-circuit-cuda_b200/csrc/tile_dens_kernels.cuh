@@ -316,15 +316,19 @@ inline const char* Circuit::run_seed_group(const DensGroup& g, const std::vector
 }
 
 // The densities plan_.steps[first..last] belong to one program point: group them into tiled sweeps
-// (singletons and the per-instruction executor keep the streaming kernels).
+// (singletons and the per-instruction executor keep the streaming kernels; k-qubit densities have sweeps of
+// their own, dens_k_kernels.cuh).
 inline const char* Circuit::run_dens_run(size_t first, size_t last, const std::vector<long>& dslot) {
+  std::vector<int> which;
+  for (size_t k = first; k <= last; k++) {
+    if (plan_.steps[k].nk > 0) QDC_TRY(dens_k(plan_.steps[k]));
+    else which.push_back((int)k);
+  }
   const qdc::SchedOptions so = base_options();
-  if (!opt_batch_dens_ || so.tile_bits == 0 || last == first) {
-    for (size_t k = first; k <= last; k++) QDC_TRY(dens_single(plan_.steps[k], dslot));
+  if (!opt_batch_dens_ || so.tile_bits == 0 || which.size() <= 1) {
+    for (int k : which) QDC_TRY(dens_single(plan_.steps[k], dslot));
     return nullptr;
   }
-  std::vector<int> which;
-  for (size_t k = first; k <= last; k++) which.push_back((int)k);
   for (const DensGroup& g : group_densities(plan_.steps, which, so.tile_bits, so.low_bits)) {
     if (g.steps.size() == 1) QDC_TRY(dens_single(plan_.steps[g.steps[0]], dslot));
     else QDC_TRY(run_dens_group(g, dslot));
@@ -334,8 +338,15 @@ inline const char* Circuit::run_dens_run(size_t first, size_t last, const std::v
 
 inline const char* Circuit::run_seed_run(size_t first, size_t last, const std::vector<const cplx_t*>& dp, bool* live) {
   std::vector<int> which;  // differentiable densities only, in reverse program order like the reference
-  for (size_t k = last + 1; k-- > first;)
-    if (kind_is_diff_dens(insts_[plan_.steps[k].inst].kind)) which.push_back((int)k);
+  for (size_t k = last + 1; k-- > first;) {
+    if (!kind_is_diff_dens(insts_[plan_.steps[k].inst].kind)) continue;
+    if (plan_.steps[k].nk > 0) {   // k-qubit densities: a seed sweep each
+      QDC_TRY(seed_k(plan_.steps[k], *live));
+      *live = true;
+    } else {
+      which.push_back((int)k);
+    }
+  }
   if (which.empty()) return nullptr;
   const qdc::SchedOptions so = base_options();
   if (!opt_batch_dens_ || so.tile_bits == 0 || which.size() == 1) {

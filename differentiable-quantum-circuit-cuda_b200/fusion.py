@@ -37,15 +37,15 @@ from typing import Callable, Dict, List, Sequence
 import numpy as np
 
 from .quantum_differentiable_circuit import (CONST_Q1, CONST_Q1_NONU, CONST_Q2, CONST_Q2_DIAG, CONST_Q2_NONU,
-                                             DIFF_Q1_DENS, DIFF_Q2_DENS, Q1_DENS, Q2_DENS, VAR_Q1, VAR_Q1_NONU,
-                                             VAR_Q2, VAR_Q2_DIAG, VAR_Q2_NONU, Circuit)
+                                             DENS_K, DIFF_DENS_K, DIFF_Q1_DENS, DIFF_Q2_DENS, Q1_DENS, Q2_DENS,
+                                             VAR_Q1, VAR_Q1_NONU, VAR_Q2, VAR_Q2_DIAG, VAR_Q2_NONU, Circuit)
 
 _Q1 = (CONST_Q1, CONST_Q1_NONU, VAR_Q1, VAR_Q1_NONU)
 _Q2D = (CONST_Q2, VAR_Q2, CONST_Q2_NONU, VAR_Q2_NONU)
 _DIAG = (CONST_Q2_DIAG, VAR_Q2_DIAG)
 _VAR = (VAR_Q2, VAR_Q2_NONU, VAR_Q2_DIAG, VAR_Q1, VAR_Q1_NONU)
 _NONU = (CONST_Q2_NONU, VAR_Q2_NONU, CONST_Q1_NONU, VAR_Q1_NONU)
-_DENS = (Q2_DENS, Q1_DENS, DIFF_Q2_DENS, DIFF_Q1_DENS)
+_DENS = (Q2_DENS, Q1_DENS, DIFF_Q2_DENS, DIFF_Q1_DENS, DENS_K, DIFF_DENS_K)
 _SWAP = np.array([0, 2, 1, 3])  # index 2 b_hi + b_lo with the two bits exchanged
 
 # how a member sits inside its fused gate
@@ -183,6 +183,20 @@ class FusedCircuit(Circuit):
         self._kinds.append(kind)
         self._inner = None
 
+    def _add_dens_k(self, positions, with_grad):
+        if any(p < 0 for p in positions):
+            raise OverflowError("can't convert negative int to unsigned")
+        if not 1 <= len(positions) <= 6:
+            raise ValueError("the number of density qubits must be in 1..6.")
+        if any(p >= self.qubits_number for p in positions):
+            raise ValueError("pos is out of the bound.")
+        if len(set(positions)) != len(positions):
+            raise ValueError("positions must be different.")
+        kind = DIFF_DENS_K if with_grad else DENS_K
+        self._program.append((kind, tuple(positions)))   # a barrier like every density (plan_fusion)
+        self._kinds.append(kind)
+        self._inner = None
+
     def __del__(self):
         pass
 
@@ -224,13 +238,15 @@ class FusedCircuit(Circuit):
 
     def _count(self, what):
         """Counts of the USER's program (not of the fused one), like Circuit._count."""
-        dens_len = lambda k: 4 if k in (Q1_DENS, DIFF_Q1_DENS) else 16            # noqa: E731
+        def dens_len(inst):
+            k = inst[0]
+            return 4 ** len(inst[1]) if k in (DENS_K, DIFF_DENS_K) else 4 if k in (Q1_DENS, DIFF_Q1_DENS) else 16
         gate_len = lambda k: 16 if k in (CONST_Q2, VAR_Q2, CONST_Q2_NONU, VAR_Q2_NONU) else 4   # noqa: E731
-        ks = self._kinds
-        diff = (DIFF_Q1_DENS, DIFF_Q2_DENS)
+        ks, prog = self._kinds, self._program
+        diff = (DIFF_Q1_DENS, DIFF_Q2_DENS, DIFF_DENS_K)
         return [len(ks), sum(k not in _DENS and k not in _VAR for k in ks), sum(k in _VAR for k in ks),
-                sum(k in _DENS for k in ks), sum(k in diff for k in ks), sum(dens_len(k) for k in ks if k in _DENS),
-                sum(dens_len(k) for k in ks if k in diff), sum(gate_len(k) for k in ks if k in _VAR)][what]
+                sum(k in _DENS for k in ks), sum(k in diff for k in ks), sum(dens_len(i) for i in prog if i[0] in _DENS),
+                sum(dens_len(i) for i in prog if i[0] in diff), sum(gate_len(k) for k in ks if k in _VAR)][what]
 
     @property
     def fused_gate_count(self) -> int:
@@ -255,12 +271,15 @@ class FusedCircuit(Circuit):
                   VAR_Q2_DIAG: "add_q2_var_gate_diag", CONST_Q1: "add_q1_const_gate",
                   CONST_Q1_NONU: "add_q1_const_gate_nonu", VAR_Q1: "add_q1_var_gate", VAR_Q1_NONU: "add_q1_var_gate_nonu",
                   Q2_DENS: "get_q2_dens_op", Q1_DENS: "get_q1_dens_op", DIFF_Q2_DENS: "get_q2_dens_op_with_grad",
-                  DIFF_Q1_DENS: "get_q1_dens_op_with_grad"}
+                  DIFF_Q1_DENS: "get_q1_dens_op_with_grad", DENS_K: "get_dens_op", DIFF_DENS_K: "get_dens_op_with_grad"}
         self._xkinds = []
         for t, x in self._exec:
             if t == "dens":
                 inst = prog[x]
-                getattr(inner, adders[inst[0]])(*inst[1:])
+                if inst[0] in (DENS_K, DIFF_DENS_K):
+                    getattr(inner, adders[inst[0]])(list(inst[1]))
+                else:
+                    getattr(inner, adders[inst[0]])(*inst[1:])
             else:
                 k = _fused_kind(x, prog)
                 self._xkinds.append(k)

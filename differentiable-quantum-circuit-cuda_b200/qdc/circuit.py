@@ -165,6 +165,9 @@ class AutoGradCircuit:
     def get_q1_dens_op(self, pos: int): self.circuit.get_q1_dens_op(pos)
     def get_q2_dens_op_with_grad(self, pos2: int, pos1: int): self.circuit.get_q2_dens_op_with_grad(pos2, pos1)
     def get_q1_dens_op_with_grad(self, pos: int): self.circuit.get_q1_dens_op_with_grad(pos)
+    # densities on 1..6 qubits, positions[0] the most significant bit (Circuit.get_dens_op)
+    def get_dens_op(self, positions): self.circuit.get_dens_op(positions)
+    def get_dens_op_with_grad(self, positions): self.circuit.get_dens_op_with_grad(positions)
 
     def build(self) -> Tuple[Callable, Callable]:
         """Returns (simple_run, autodiff_run), src/qdc/circuit.py:160-202.

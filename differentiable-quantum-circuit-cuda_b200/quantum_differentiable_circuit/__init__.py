@@ -24,9 +24,9 @@ import numpy as np
 
 from .._ffi import Lib, ProfileEntry, QdcError, Stats, default_precision, get_lib
 
-# enum Instruction, src/circuit.rs:53-68
+# enum Instruction, src/circuit.rs:53-68, then the densities on 3..6 qubits (include/qdc_circuit.h)
 (CONST_Q2, VAR_Q2, CONST_Q2_NONU, VAR_Q2_NONU, CONST_Q2_DIAG, VAR_Q2_DIAG, CONST_Q1, CONST_Q1_NONU, VAR_Q1,
- VAR_Q1_NONU, Q2_DENS, Q1_DENS, DIFF_Q2_DENS, DIFF_Q1_DENS) = range(14)
+ VAR_Q1_NONU, Q2_DENS, Q1_DENS, DIFF_Q2_DENS, DIFF_Q1_DENS, DENS_K, DIFF_DENS_K) = range(16)
 
 (N_INSTRUCTIONS, N_CONST_GATES, N_VAR_GATES, N_DENSITIES, N_DIFF_DENSITIES, RUN_OUT_LEN, FORWARD_OUT_LEN,
  BACKWARD_OUT_LEN) = range(8)
@@ -40,6 +40,7 @@ class Circuit:
         self._lib.call("qdc_circuit_new", C.byref(h), self.qubits_number)
         self._h = h
         self._kinds: List[int] = []
+        self._dims: List[int] = []   # side of every instruction's density output (0: a gate)
 
     def __del__(self):
         try:
@@ -66,6 +67,15 @@ class Circuit:
             raise OverflowError("can't convert negative int to unsigned")
         self._lib.call("qdc_circuit_add", self._h, kind, pos2, pos1)
         self._kinds.append(kind)
+        self._dims.append(2 if kind in (Q1_DENS, DIFF_Q1_DENS) else 4 if kind in (Q2_DENS, DIFF_Q2_DENS) else 0)
+
+    def _add_dens_k(self, positions: List[int], with_grad: bool):
+        if any(p < 0 for p in positions):
+            raise OverflowError("can't convert negative int to unsigned")
+        pos = np.array(positions, dtype=np.uintp)
+        self._lib.call("qdc_circuit_add_dens", self._h, pos.ctypes.data, pos.size, int(with_grad))
+        self._kinds.append(DIFF_DENS_K if with_grad else DENS_K)
+        self._dims.append(1 << pos.size)
 
     def add_q2_const_gate(self, pos2: int, pos1: int): self._add(CONST_Q2, pos2, pos1)
     def add_q2_const_gate_diag(self, pos2: int, pos1: int): self._add(CONST_Q2_DIAG, pos2, pos1)
@@ -81,6 +91,25 @@ class Circuit:
     def get_q1_dens_op(self, pos: int): self._add(Q1_DENS, pos)
     def get_q2_dens_op_with_grad(self, pos2: int, pos1: int): self._add(DIFF_Q2_DENS, pos2, pos1)
     def get_q1_dens_op_with_grad(self, pos: int): self._add(DIFF_Q1_DENS, pos)
+
+    def get_dens_op(self, positions: Sequence[int]):
+        """Reduced density matrix on the qubits `positions` = [p_{k-1}, ..., p_0] (1 <= k <= 6, distinct, any order):
+        rho[r, c] = sum_rest psi[r, rest] conj psi[c, rest], shape (2^k, 2^k), positions[0] the most significant bit
+        of r and c.  k = 1 and 2 are get_q1_dens_op(p) and get_q2_dens_op(p2, p1)."""
+        self._add_dens(positions, False)
+
+    def get_dens_op_with_grad(self, positions: Sequence[int]):
+        """`get_dens_op` with gradient: forward returns it, backward takes its (2^k, 2^k) cotangent."""
+        self._add_dens(positions, True)
+
+    def _add_dens(self, positions, with_grad: bool):
+        pos = [int(p) for p in positions]
+        if len(pos) == 1:
+            (self.get_q1_dens_op_with_grad if with_grad else self.get_q1_dens_op)(pos[0])
+        elif len(pos) == 2:
+            (self.get_q2_dens_op_with_grad if with_grad else self.get_q2_dens_op)(pos[0], pos[1])
+        else:
+            self._add_dens_k(pos, with_grad)
 
     # ---- marshalling ----
     def _flatten(self, arrays: Sequence, ndim: int):
@@ -109,9 +138,8 @@ class Circuit:
         self._lib.call(name, self._h, cf.ctypes.data, cl.ctypes.data, cl.size, vf.ctypes.data, vl.ctypes.data,
                        vl.size, out.ctypes.data, cap, C.byref(n_out))
         res, o = [], 0
-        for k in self._kinds:
+        for k, m in zip(self._kinds, self._dims):
             if k in dens_kinds:
-                m = 2 if k in (Q1_DENS, DIFF_Q1_DENS) else 4
                 res.append(out[o:o + m * m].reshape(m, m).copy())
                 o += m * m
         assert o == n_out.value
@@ -120,12 +148,12 @@ class Circuit:
     # ---- src/circuit.rs:164-212 ----
     def run(self, const_gates, var_gates) -> List[np.ndarray]:
         return self._sweep("qdc_circuit_run", const_gates, var_gates, RUN_OUT_LEN,
-                           (Q1_DENS, Q2_DENS, DIFF_Q1_DENS, DIFF_Q2_DENS))
+                           (Q1_DENS, Q2_DENS, DIFF_Q1_DENS, DIFF_Q2_DENS, DENS_K, DIFF_DENS_K))
 
     # ---- src/circuit.rs:214-264 ----
     def forward(self, const_gates, var_gates) -> List[np.ndarray]:
         return self._sweep("qdc_circuit_forward", const_gates, var_gates, FORWARD_OUT_LEN,
-                           (DIFF_Q1_DENS, DIFF_Q2_DENS))
+                           (DIFF_Q1_DENS, DIFF_Q2_DENS, DIFF_DENS_K))
 
     # ---- src/circuit.rs:266-429 ----
     def backward(self, grads_wrt_density, const_gates, var_gates) -> List[np.ndarray]:

@@ -40,6 +40,7 @@ class ShardedCircuit(Circuit):
                        uid.ctypes.data)
         self._h = h
         self._kinds = []
+        self._dims = []
 
     @property
     def peer_exchange(self) -> bool:

@@ -30,12 +30,14 @@ extern "C" {
 
 typedef struct qdc_circuit qdc_circuit;
 
-/* Instruction kinds == `enum Instruction`, src/circuit.rs:53-68 (same order). */
+/* Instruction kinds == `enum Instruction`, src/circuit.rs:53-68 (same order),
+ * then the densities on 3..6 qubits, which only qdc_circuit_add_dens adds. */
 enum qdc_kind {
   QDC_CONST_Q2 = 0, QDC_VAR_Q2 = 1, QDC_CONST_Q2_NONU = 2, QDC_VAR_Q2_NONU = 3,
   QDC_CONST_Q2_DIAG = 4, QDC_VAR_Q2_DIAG = 5,
   QDC_CONST_Q1 = 6, QDC_CONST_Q1_NONU = 7, QDC_VAR_Q1 = 8, QDC_VAR_Q1_NONU = 9,
-  QDC_Q2_DENS = 10, QDC_Q1_DENS = 11, QDC_DIFF_Q2_DENS = 12, QDC_DIFF_Q1_DENS = 13
+  QDC_Q2_DENS = 10, QDC_Q1_DENS = 11, QDC_DIFF_Q2_DENS = 12, QDC_DIFF_Q1_DENS = 13,
+  QDC_DENS_K = 14, QDC_DIFF_DENS_K = 15
 };
 
 /* qdc_circuit_count selectors */
@@ -70,8 +72,16 @@ int qdc_circuit_peer_exchange(const qdc_circuit* c);
 const char* qdc_circuit_free(qdc_circuit* c);
 /* Circuit::set_state_from_vector, src/circuit.rs:104-106 */
 const char* qdc_circuit_set_state_from_host(qdc_circuit* c, const qdc_complex* host_state, size_t len);
-/* The 14 builder methods, src/circuit.rs:108-162.  pos1 is ignored for q1 kinds. */
+/* The 14 builder methods, src/circuit.rs:108-162.  pos1 is ignored for q1 kinds.
+ * QDC_DENS_K / QDC_DIFF_DENS_K are refused here (they need qdc_circuit_add_dens). */
 const char* qdc_circuit_add(qdc_circuit* c, int kind, size_t pos2, size_t pos1);
+/* Reduced density matrix on k = 1..6 distinct qubits positions[0..k-1] (positions[0] is the most
+ * significant bit of the row and column index), with gradient if `with_grad`:
+ *   rho[r, c] = sum_rest psi[r, rest] conj psi[c, rest],   2^k x 2^k, row-major, not normalised.
+ * k = 1 and 2 add QDC_(DIFF_)Q1_DENS(positions[0]) and QDC_(DIFF_)Q2_DENS(positions[0], positions[1]);
+ * k >= 3 adds QDC_(DIFF_)DENS_K.  Like every density it is a barrier; run / forward return it in program
+ * order and backward takes its (conjugated) 4^k-entry cotangent in program order. */
+const char* qdc_circuit_add_dens(qdc_circuit* c, const size_t* positions, size_t k, int with_grad);
 size_t qdc_circuit_count(const qdc_circuit* c, int what);
 
 /* Circuit::run, src/circuit.rs:164-212 (all densities, program order). */
