@@ -27,20 +27,25 @@ enum Kind {
   K_CONST_Q2 = 0, K_VAR_Q2, K_CONST_Q2_NONU, K_VAR_Q2_NONU, K_CONST_Q2_DIAG, K_VAR_Q2_DIAG,
   K_CONST_Q1, K_CONST_Q1_NONU, K_VAR_Q1, K_VAR_Q1_NONU,
   K_Q2_DENS, K_Q1_DENS, K_DIFF_Q2_DENS, K_DIFF_Q1_DENS,
-  K_DENS_K, K_DIFF_DENS_K   // densities on 3..6 qubits (add_dens; dens_k_kernels.cuh)
+  K_DENS_K, K_DIFF_DENS_K,  // densities on 3..6 qubits (add_dens; dens_k_kernels.cuh)
+  K_CONST_GATE_K, K_VAR_GATE_K, K_CONST_GATE_K_NONU, K_VAR_GATE_K_NONU   // gates on 3..6 qubits (add_gate; gate_k_kernels.cuh)
 };
 
+// one- and two-qubit gates (the k-qubit gates are kind_is_k_gate)
 static inline bool kind_is_gate(int k) { return k <= K_VAR_Q1_NONU; }
 static inline bool kind_is_var(int k) {
-  return k == K_VAR_Q2 || k == K_VAR_Q2_NONU || k == K_VAR_Q2_DIAG || k == K_VAR_Q1 || k == K_VAR_Q1_NONU;
+  return k == K_VAR_Q2 || k == K_VAR_Q2_NONU || k == K_VAR_Q2_DIAG || k == K_VAR_Q1 || k == K_VAR_Q1_NONU ||
+         k == K_VAR_GATE_K || k == K_VAR_GATE_K_NONU;
 }
 static inline bool kind_is_nonu(int k) {
-  return k == K_CONST_Q2_NONU || k == K_VAR_Q2_NONU || k == K_CONST_Q1_NONU || k == K_VAR_Q1_NONU;
+  return k == K_CONST_Q2_NONU || k == K_VAR_Q2_NONU || k == K_CONST_Q1_NONU || k == K_VAR_Q1_NONU ||
+         k == K_CONST_GATE_K_NONU || k == K_VAR_GATE_K_NONU;
 }
 static inline bool kind_is_diag(int k) { return k == K_CONST_Q2_DIAG || k == K_VAR_Q2_DIAG; }
 static inline bool kind_is_q1(int k) { return k >= K_CONST_Q1 && k <= K_VAR_Q1_NONU; }
 static inline bool kind_is_q2dense(int k) { return k <= K_VAR_Q2_NONU; }
-static inline bool kind_is_dens(int k) { return k >= K_Q2_DENS; }
+static inline bool kind_is_dens(int k) { return k >= K_Q2_DENS && k <= K_DIFF_DENS_K; }
+static inline bool kind_is_k_gate(int k) { return k >= K_CONST_GATE_K && k <= K_VAR_GATE_K_NONU; }
 static inline bool kind_is_diff_dens(int k) { return k == K_DIFF_Q2_DENS || k == K_DIFF_Q1_DENS || k == K_DIFF_DENS_K; }
 static inline bool kind_is_k_dens(int k) { return k == K_DENS_K || k == K_DIFF_DENS_K; }
 static inline bool kind_is_q1_dens(int k) { return k == K_Q1_DENS || k == K_DIFF_Q1_DENS; }
@@ -50,13 +55,18 @@ static inline int kind_dens_len(int k) { return kind_is_q1_dens(k) ? 4 : 16; }
 struct Inst {
   int kind;
   int pos2, pos1;  // q1 kinds use pos2 only
-  int nk = 0;      // k-qubit densities: the qubits kpos[0..nk-1], most significant first (pos2 = pos1 = -1)
+  int nk = 0;      // k-qubit densities and gates: the qubits kpos[0..nk-1], most significant first (pos2 = pos1 = -1)
   int kpos[6] = {-1, -1, -1, -1, -1, -1};
 };
 
 // complex entries of a density's output / cotangent
 static inline size_t dens_len(const Inst& in) {
   return kind_is_k_dens(in.kind) ? (size_t)1 << (2 * in.nk) : (size_t)kind_dens_len(in.kind);
+}
+
+// complex entries of a gate's matrix / gradient
+static inline size_t gate_len(const Inst& in) {
+  return kind_is_k_gate(in.kind) ? (size_t)1 << (2 * in.nk) : (size_t)kind_gate_len(in.kind);
 }
 
 struct Stats {
@@ -79,11 +89,12 @@ struct GateList {
 // (enabled by option "profile"); feeds bench.py's roofline block.
 enum ProfCat {
   CAT_FWD_Q1 = 0, CAT_FWD_Q2, CAT_FWD_DIAG, CAT_DENSITY, CAT_SEED, CAT_UNCOMPUTE, CAT_REV_Q1, CAT_REV_Q2,
-  CAT_REV_DIAG, CAT_REV_CONST, CAT_TILE_FWD, CAT_TILE_BWD, CAT_EXCHANGE, CAT_TC_FWD, CAT_TC_BWD, CAT_COUNT
+  CAT_REV_DIAG, CAT_REV_CONST, CAT_TILE_FWD, CAT_TILE_BWD, CAT_EXCHANGE, CAT_TC_FWD, CAT_TC_BWD, CAT_GATE_K_FWD,
+  CAT_GATE_K_REV, CAT_COUNT
 };
 static const char* const kProfCatNames[CAT_COUNT] = {
     "fwd_q1", "fwd_q2", "fwd_diag", "density", "seed", "uncompute", "rev_q1", "rev_q2",
-    "rev_diag", "rev_const", "tile_fwd", "tile_bwd", "exchange", "tc_fwd", "tc_bwd"};
+    "rev_diag", "rev_const", "tile_fwd", "tile_bwd", "exchange", "tc_fwd", "tc_bwd", "gate_k_fwd", "gate_k_rev"};
 
 struct ProfEntry {
   uint64_t launches = 0;
@@ -297,6 +308,9 @@ class Circuit {
   size_t d_kmat_cap_ = 0;
   std::vector<cplx_t> h_kmat_;
   std::vector<size_t> kmat_ofs_;
+  // k-qubit gates: their device forms share the cotangents' region and copy (at gmat_ofs_[instruction]); the
+  // gradients of the variable ones follow the 32-double slots in d_res_ (at kgofs_[instruction], in doubles)
+  std::vector<size_t> gmat_ofs_, kgofs_;
   cudaStream_t stream_ = 0;
   Stats stats_;
   int opt_fuse_ = 2;          // 0: one pass per instruction, 1: tiled multi-gate passes, 2: + register-blocked forward
@@ -477,6 +491,7 @@ class Circuit {
 
   const char* add(int kind, size_t pos2, size_t pos1) {
     if (kind_is_k_dens(kind)) return qdc_errf("kind %d carries its qubits through qdc_circuit_add_dens.", kind);
+    if (kind_is_k_gate(kind)) return qdc_errf("kind %d carries its qubits through qdc_circuit_add_gate.", kind);
     if (kind < 0 || kind > K_DIFF_Q1_DENS) return qdc_errf("Unknown instruction kind %d.", kind);
     const bool one = kind_is_q1(kind) || kind_is_q1_dens(kind);
     if (one) {
@@ -510,19 +525,44 @@ class Circuit {
     return nullptr;
   }
 
+  // Gate on k = 1..6 qubits, positions[0] the most significant bit of its row and column index; k <= 2 adds the
+  // one- and two-qubit kinds.
+  const char* add_gate(const size_t* positions, size_t k, bool variable, bool non_unitary) {
+    if (k < 1 || k > 6) return qdc_errf("the number of gate qubits must be in 1..6, got %zu.", k);
+    if (k == 1)
+      return add(variable ? (non_unitary ? K_VAR_Q1_NONU : K_VAR_Q1) : (non_unitary ? K_CONST_Q1_NONU : K_CONST_Q1),
+                 positions[0], 0);
+    if (k == 2)
+      return add(variable ? (non_unitary ? K_VAR_Q2_NONU : K_VAR_Q2) : (non_unitary ? K_CONST_Q2_NONU : K_CONST_Q2),
+                 positions[0], positions[1]);
+    Inst in{variable ? (non_unitary ? K_VAR_GATE_K_NONU : K_VAR_GATE_K)
+                     : (non_unitary ? K_CONST_GATE_K_NONU : K_CONST_GATE_K), -1, -1};
+    for (size_t j = 0; j < k; j++) {
+      if (positions[j] >= (size_t)n_) return qdc_errf("pos is out of the bound.");
+      for (size_t i = 0; i < j; i++)
+        if (positions[i] == positions[j]) return qdc_errf("positions must be different.");
+      in.kpos[j] = (int)positions[j];
+    }
+    in.nk = (int)k;
+    insts_.push_back(in);
+    forward_valid_ = false;
+    return nullptr;
+  }
+
   size_t count(int what) const {
     size_t c = 0;
     for (const Inst& in : insts_) {
       const int k = in.kind;
+      const bool gate = kind_is_gate(k) || kind_is_k_gate(k);
       switch (what) {
         case 0: c++; break;
-        case 1: c += kind_is_gate(k) && !kind_is_var(k); break;
-        case 2: c += kind_is_gate(k) && kind_is_var(k); break;
+        case 1: c += gate && !kind_is_var(k); break;
+        case 2: c += gate && kind_is_var(k); break;
         case 3: c += kind_is_dens(k); break;
         case 4: c += kind_is_diff_dens(k); break;
         case 5: c += kind_is_dens(k) ? dens_len(in) : 0; break;
         case 6: c += kind_is_diff_dens(k) ? dens_len(in) : 0; break;
-        case 7: c += (kind_is_gate(k) && kind_is_var(k)) ? kind_gate_len(k) : 0; break;
+        case 7: c += (gate && kind_is_var(k)) ? gate_len(in) : 0; break;
       }
     }
     return c;
@@ -536,7 +576,7 @@ class Circuit {
     size_t ci = 0, vi = 0, coff = 0, voff = 0;
     for (size_t i = 0; i < insts_.size(); i++) {
       const int k = insts_[i].kind;
-      if (!kind_is_gate(k)) continue;
+      if (!kind_is_gate(k) && !kind_is_k_gate(k)) continue;
       const bool var = kind_is_var(k);
       const GateList& gl = var ? vg : cg;
       size_t& idx = var ? vi : ci;
@@ -545,7 +585,7 @@ class Circuit {
         if (backward) return qdc_errf("The number of gates is less than required.");
         return qdc_errf("The number of %s gates is less than required.", var ? "variable" : "constant");
       }
-      if ((int)gl.lens[idx] != kind_gate_len(k)) return qdc_errf("Incorrect len of the gate's buffer.");
+      if ((size_t)gl.lens[idx] != gate_len(insts_[i])) return qdc_errf("Incorrect len of the gate's buffer.");
       ptr[i] = gl.flat + off;
       off += gl.lens[idx];
       idx++;
@@ -698,6 +738,7 @@ class Circuit {
     if (kind_is_q2dense(k)) return 1;
     if (kind_is_diag(k)) return 2;
     if (kind_is_k_dens(k)) return 5;
+    if (kind_is_k_gate(k)) return 6;
     return kind_is_q1_dens(k) ? 3 : 4;
   }
 
@@ -1053,6 +1094,9 @@ class Circuit {
       d_kres_cap_ = nkres;
     }
     h_kres_.resize(nkres);
+    h_kmat_.clear();
+    QDC_TRY(add_gate_k_forms(gp, false));
+    QDC_TRY(upload_kmat());
     forward_valid_ = false;
     build_plan(all_dens);
     if (!plan_.ok)
@@ -1173,6 +1217,9 @@ class Circuit {
           si = sj;
           break;
         }
+        case qdc::ST_GATE_K:
+          QDC_TRY(gate_k_apply(st, state_, d_kmat_ + gmat_ofs_[st.inst], CAT_GATE_K_FWD));
+          break;
       }
     }
     return nullptr;
@@ -1197,6 +1244,32 @@ class Circuit {
            eng_seed_q2(stream_, ws_, state_, bwd_, dp[st.inst], st.p2, st.p1, n_loc_, live));
     }
     account(1, 1, live ? 3 : 2);
+    return nullptr;
+  }
+
+  // Appends the device forms of every k-qubit gate (gate_k_forms) to h_kmat_, at gmat_ofs_[instruction].
+  const char* add_gate_k_forms(const std::vector<const cplx_t*>& gp, bool reverse) {
+    gmat_ofs_.assign(insts_.size(), 0);
+    for (size_t i = 0; i < insts_.size(); i++) {
+      const Inst& in = insts_[i];
+      if (!kind_is_k_gate(in.kind)) continue;
+      gmat_ofs_[i] = h_kmat_.size();
+      QDC_TRY(gate_k_forms(gp[i], in.nk, kind_is_nonu(in.kind), reverse, &h_kmat_));
+    }
+    return nullptr;
+  }
+
+  // h_kmat_ -> d_kmat_, one copy per call
+  const char* upload_kmat() {
+    if (h_kmat_.empty()) return nullptr;
+    if (h_kmat_.size() > d_kmat_cap_) {
+      if (d_kmat_) QDC_CUDA(cudaFree(d_kmat_));
+      d_kmat_ = nullptr;
+      QDC_CUDA(cudaMalloc((void**)&d_kmat_, h_kmat_.size() * sizeof(cplx_t)));
+      d_kmat_cap_ = h_kmat_.size();
+    }
+    QDC_CUDA(cudaMemcpyAsync(d_kmat_, h_kmat_.data(), h_kmat_.size() * sizeof(cplx_t), cudaMemcpyHostToDevice,
+                             stream_));
     return nullptr;
   }
 
@@ -1237,39 +1310,36 @@ class Circuit {
       kmat_ofs_[i] = h_kmat_.size();
       h_kmat_.insert(h_kmat_.end(), dp[i], dp[i] + dens_len(insts_[i]));
     }
+    QDC_TRY(add_gate_k_forms(gp, true));
     const size_t need = count(7);
     if (cap < need) return qdc_errf("Output buffer too small: %zu < %zu.", cap, need);
-    const size_t nvar = count(2);
-    QDC_TRY(ensure_results(nvar));
-    if (nvar) QDC_CUDA(cudaMemsetAsync(d_res_, 0, nvar * 32 * sizeof(double), stream_));
-    if (!bwd_) QDC_CUDA(cudaMalloc((void**)&bwd_, bytes()));  // (sharded mode allocated it in shard())
-    if (!h_kmat_.empty()) {
-      if (h_kmat_.size() > d_kmat_cap_) {
-        if (d_kmat_) QDC_CUDA(cudaFree(d_kmat_));
-        d_kmat_ = nullptr;
-        QDC_CUDA(cudaMalloc((void**)&d_kmat_, h_kmat_.size() * sizeof(cplx_t)));
-        d_kmat_cap_ = h_kmat_.size();
-      }
-      QDC_CUDA(cudaMemcpyAsync(d_kmat_, h_kmat_.data(), h_kmat_.size() * sizeof(cplx_t), cudaMemcpyHostToDevice,
-                               stream_));
-    }
-
-    // variable-gate slot of every instruction
+    // variable-gate slot of every one- and two-qubit instruction
     std::vector<long> vslot(insts_.size(), -1);
     {
       long s = 0;
       for (size_t i = 0; i < insts_.size(); i++)
         if (kind_is_gate(insts_[i].kind) && kind_is_var(insts_[i].kind)) vslot[i] = s++;
     }
+    const size_t nvar = (size_t)std::count_if(vslot.begin(), vslot.end(), [](long s) { return s >= 0; });
+    // gradients of the variable k-qubit gates: 2 * 4^k doubles each, after the slots
+    size_t ndbl = nvar * 32;
+    kgofs_.assign(insts_.size(), 0);
+    for (size_t i = 0; i < insts_.size(); i++) {
+      if (!kind_is_k_gate(insts_[i].kind) || !kind_is_var(insts_[i].kind)) continue;
+      kgofs_[i] = ndbl;
+      ndbl += 2 * gate_len(insts_[i]);
+    }
+    QDC_TRY(ensure_results((ndbl + 31) / 32));
+    if (ndbl) QDC_CUDA(cudaMemsetAsync(d_res_, 0, ndbl * sizeof(double), stream_));
+    if (!bwd_) QDC_CUDA(cudaMalloc((void**)&bwd_, bytes()));  // (sharded mode allocated it in shard())
+    QDC_TRY(upload_kmat());
 #ifndef QDC_F64
     QDC_TRY(tc_begin(true));
 #endif
     QDC_TRY(run_backward(gp, dp, vslot));
     cur_map_.clear();  // every swap has been replayed in reverse: identity layout again
-    if (nvar) {
-      QDC_CUDA(cudaMemcpyAsync(h_res_.data(), d_res_, nvar * 32 * sizeof(double), cudaMemcpyDeviceToHost,
-                               stream_));
-    }
+    if (ndbl)
+      QDC_CUDA(cudaMemcpyAsync(h_res_.data(), d_res_, ndbl * sizeof(double), cudaMemcpyDeviceToHost, stream_));
     QDC_CUDA(cudaStreamSynchronize(stream_));
     if (prof_.on) prof_.collect();
 #ifndef QDC_F64
@@ -1277,8 +1347,18 @@ class Circuit {
 #endif
     size_t o = 0;
     for (size_t i = 0; i < insts_.size(); i++) {
-      if (vslot[i] < 0) continue;
       const Inst& in = insts_[i];
+      if (kind_is_k_gate(in.kind) && kind_is_var(in.kind)) {
+        const size_t len = gate_len(in);
+        const double* h = &h_res_[kgofs_[i]];
+        for (size_t j = 0; j < len; j++) {
+          out[o + j].x = (real_t)h[2 * j];
+          out[o + j].y = (real_t)h[2 * j + 1];
+        }
+        o += len;
+        continue;
+      }
+      if (vslot[i] < 0) continue;
 #ifndef QDC_F64
       if (const std::vector<zc>* tg = tc_gradient(i)) {   // gate of a tensor-core block: already in reference order
         for (size_t j = 0; j < tg->size(); j++) {
@@ -1370,6 +1450,15 @@ class Circuit {
         case qdc::ST_GATE:
           QDC_TRY(bwd_gate_step(st, gp, vslot, live));
           break;
+        case qdc::ST_GATE_K: {
+          // no adjoint yet: un-compute only; a variable gate keeps its zero gradient
+          const cplx_t* inv = d_kmat_ + gmat_ofs_[st.inst];
+          const int k = insts_[st.inst].kind;
+          if (!live) QDC_TRY(gate_k_apply(st, state_, inv, CAT_GATE_K_REV));
+          else QDC_TRY(gate_k_reverse(st, inv, inv + ((size_t)1 << (2 * st.nk)),
+                                      kind_is_var(k) ? d_res_ + kgofs_[st.inst] : nullptr));
+          break;
+        }
         case qdc::ST_TILE:
 #ifndef QDC_F64
           if (tc_step_ok(st)) {
@@ -1469,6 +1558,13 @@ class Circuit {
   template <int KQ> const char* launch_seed_k(const DensKParams& p, const cplx_t* G);
   const char* dens_k(const qdc::Step& st);
   const char* seed_k(const qdc::Step& st, bool live);
+  // k-qubit gates (gate_k_kernels.cuh)
+  const char* gate_k_forms(const cplx_t* U, int nk, bool nonu, bool reverse, std::vector<cplx_t>* h);
+  template <int KQ> const char* launch_gate_k(const DensKParams& p, cplx_t* buf, const cplx_t* At);
+  template <int KQ> const char* launch_gate_k_rev(const DensKParams& p, const cplx_t* At, const cplx_t* Bt,
+                                                  double* gdst);
+  const char* gate_k_apply(const qdc::Step& st, cplx_t* buf, const cplx_t* At, int cat);
+  const char* gate_k_reverse(const qdc::Step& st, const cplx_t* At, const cplx_t* Bt, double* gdst);
   std::vector<char> diag_hilo_;  // diagonal gradient of this instruction came back in (hi,lo) order
   double* tile_partials_ = nullptr;
   size_t tile_partials_cap_ = 0;

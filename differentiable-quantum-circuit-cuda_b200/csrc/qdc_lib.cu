@@ -8,6 +8,7 @@
 #include "tile_rb_soa_kernels.cuh"
 #include "tile_dens_kernels.cuh"
 #include "dens_k_kernels.cuh"
+#include "gate_k_kernels.cuh"
 #include "tc_exec.cuh"
 
 struct qdc_circuit {
@@ -23,7 +24,7 @@ QDC_EXPORT const char* qdc_precision(void) {
 #endif
 }
 
-QDC_EXPORT int qdc_abi_version(void) { return 3; }
+QDC_EXPORT int qdc_abi_version(void) { return 4; }
 
 QDC_EXPORT const char* qdc_circuit_new(qdc_circuit** out, size_t qubits_number) {
   if (qubits_number < 1 || qubits_number > 40) return qdc_errf("qubits_number out of range.");
@@ -77,6 +78,11 @@ QDC_EXPORT const char* qdc_circuit_add(qdc_circuit* c, int kind, size_t pos2, si
 
 QDC_EXPORT const char* qdc_circuit_add_dens(qdc_circuit* c, const size_t* positions, size_t k, int with_grad) {
   return c->impl.add_dens(positions, k, with_grad != 0);
+}
+
+QDC_EXPORT const char* qdc_circuit_add_gate(qdc_circuit* c, const size_t* positions, size_t k, int variable,
+                                            int non_unitary) {
+  return c->impl.add_gate(positions, k, variable != 0, non_unitary != 0);
 }
 
 QDC_EXPORT size_t qdc_circuit_count(const qdc_circuit* c, int what) { return c->impl.count(what); }

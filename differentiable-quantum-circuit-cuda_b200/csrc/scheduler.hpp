@@ -11,7 +11,8 @@
 //  * Density instructions are full barriers (a Diff density must see exactly
 //    the gates that precede it in program order, otherwise the gradients of
 //    non-unitary directions change).  A k-qubit density (kind class 5) needs
-//    all its k qubits local at once.
+//    all its k qubits local at once.  So does a k-qubit gate (class 6, step
+//    ST_GATE_K), which is a full barrier too: nothing is reordered across it.
 //
 // Sharding: with 2^g ranks the top g PHYSICAL bit positions are the rank
 // index ("global").  A logical->physical qubit map is maintained; dense gates
@@ -32,7 +33,7 @@
 
 namespace qdc {
 
-enum StepType : int { ST_GATE = 0, ST_DENS = 1, ST_SWAP = 2, ST_TILE = 3 };
+enum StepType : int { ST_GATE = 0, ST_DENS = 1, ST_SWAP = 2, ST_TILE = 3, ST_GATE_K = 4 };
 
 struct Step {
   int type = ST_GATE;
@@ -42,8 +43,12 @@ struct Step {
   int first = 0, count = 0;  // TILE: range in Plan::tile_steps
   int tb_first = 0, tb_count = 0;  // TILE: range in Plan::tile_bits (sorted physical positions)
   int grp_first = 0, grp_count = 0;  // TILE: range in Plan::groups (register-block groups)
-  int nk = 0, pk[6] = {-1, -1, -1, -1, -1, -1};  // k-qubit DENS (p2 = p1 = -1): physical positions, most significant first
+  int nk = 0, pk[6] = {-1, -1, -1, -1, -1, -1};  // k-qubit DENS / GATE_K (p2 = p1 = -1): physical positions, most significant first
 };
+
+// Steps nothing may be moved across: densities and k-qubit gates.  (A k-qubit gate has p2 = p1 = -1, so it marks
+// no position dirty: treated as an ordinary deferred step, later gates on its qubits could overtake it.)
+inline bool is_wall(const Step& st) { return st.type == ST_DENS || st.type == ST_GATE_K; }
 
 // A register-block group inside a tile pass: `count` consecutive tile gates
 // (starting at Plan::tile_steps[first]) that all act within <= 4 positions.
@@ -63,10 +68,11 @@ struct Plan {
 };
 
 struct SchedInst {
-  int kind_class;  // 0: dense q1, 1: dense q2, 2: diagonal q2, 3: density q1, 4: density q2, 5: density on nq qubits
-  int q2, q1;      // logical qubits (q1 = -1 for one-qubit instructions; both -1 for class 5)
+  int kind_class;  // 0: dense q1, 1: dense q2, 2: diagonal q2, 3: density q1, 4: density q2, 5: density on nq qubits,
+                   // 6: gate on nq qubits
+  int q2, q1;      // logical qubits (q1 = -1 for one-qubit instructions; both -1 for classes 5 and 6)
   bool skip;       // densities that this sweep does not evaluate
-  int nq = 0;      // class 5: the logical qubits qk[0..nq-1], most significant first
+  int nq = 0;      // classes 5 and 6: the logical qubits qk[0..nq-1], most significant first
   int qk[6] = {-1, -1, -1, -1, -1, -1};
 };
 
@@ -130,7 +136,7 @@ class Scheduler {
   std::vector<bool> done_;
   std::vector<int> map_;  // logical -> physical
 
-  bool is_dens(const SchedInst& s) const { return s.kind_class >= 3; }
+  bool is_barrier(const SchedInst& s) const { return s.kind_class >= 3; }   // densities and k-qubit gates
   bool local(int q) const { return map_[q] < o_.n_loc; }
 
   // One sweep in program order: every instruction whose predecessors (on its
@@ -142,13 +148,13 @@ class Scheduler {
     for (int i = 0; i < N; i++) {
       if (done_[i]) continue;
       const SchedInst& s = in_[i];
-      if (is_dens(s)) {
+      if (is_barrier(s)) {
         // barrier: runs only if everything before it is done
         if (any_blocked) break;
         bool ok = s.nq > 0 || (local(s.q2) && (s.q1 < 0 || local(s.q1)));
         for (int j = 0; j < s.nq; j++) ok = ok && local(s.qk[j]);
         if (!ok) break;
-        ready.push_back(make_step(i, ST_DENS));
+        ready.push_back(make_step(i, s.kind_class == 6 ? ST_GATE_K : ST_DENS));
         done_[i] = true;
         continue;
       }
@@ -239,8 +245,8 @@ class Scheduler {
           plan.steps.push_back(st);
         } else {
           deferred.push_back(st);
-          if (st.type == ST_DENS) {
-            // densities are barriers: nothing after them may be pulled forward
+          if (is_wall(st)) {
+            // densities and k-qubit gates are barriers: nothing after them may be pulled forward
             for (int p = 0; p < o_.n; p++) dirty[p] = true;
           } else {
             if (st.p2 >= 0) dirty[st.p2] = true;
@@ -293,7 +299,7 @@ class Scheduler {
         if (chosen[k]) continue;
         const Step& st = pending[k];
         if (!tileable(st)) {
-          if (st.type == ST_DENS) break;
+          if (is_wall(st)) break;
           if (st.p2 >= 0 && st.p2 < o_.n) dirty[st.p2] = 1;
           if (st.p1 >= 0 && st.p1 < o_.n) dirty[st.p1] = 1;
           continue;
@@ -334,7 +340,7 @@ class Scheduler {
         if (chosen[k]) continue;
         const Step& st = pending[k];
         if (!tileable(st)) {
-          if (st.type == ST_DENS) { wall = true; break; }
+          if (is_wall(st)) { wall = true; break; }
           if (st.p2 >= 0 && st.p2 < o_.n) dirty[st.p2] = 1;
           if (st.p1 >= 0 && st.p1 < o_.n) dirty[st.p1] = 1;
           continue;
@@ -453,8 +459,8 @@ class Scheduler {
     std::vector<int> nu(o_.n, N + 1);
     for (int i = N - 1; i >= 0; i--) {
       if (done_[i]) continue;
-      // (the qubits of a k-qubit density share one next use: a remap for it never evicts another of them, the
-      // victims must be strictly less urgent)
+      // (the qubits of a k-qubit density or gate share one next use: a remap for it never evicts another of them,
+      // the victims must be strictly less urgent)
       for (int j = 0; j < in_[i].nq; j++) nu[in_[i].qk[j]] = i;
       if (in_[i].nq > 0) continue;
       nu[in_[i].q2] = i;

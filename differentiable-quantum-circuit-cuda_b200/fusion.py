@@ -24,6 +24,8 @@ Fusion rules (program order is preserved wherever two gates share a qubit):
   * a two-qubit gate joins the last gate on BOTH its qubits if that is one and the same two-qubit gate;
     otherwise it starts a new fused gate and absorbs the still-open ONE-qubit gates of its two qubits;
   * every density instruction closes all gates (it must see the state of its program point);
+  * a gate on 3..6 qubits (`add_const_gate(positions)` and friends) is a barrier like a density: it closes all
+    gates and runs unfused, its matrix and gradient pass through unchanged;
   * diagonal gates are taken as unitary (the reference's un-compute multiplies by conj(d),
     src/quantized_tensor.rs:153-156): a fused gate is NonU iff one of its members is.
 
@@ -36,14 +38,16 @@ from typing import Callable, Dict, List, Sequence
 
 import numpy as np
 
-from .quantum_differentiable_circuit import (CONST_Q1, CONST_Q1_NONU, CONST_Q2, CONST_Q2_DIAG, CONST_Q2_NONU,
-                                             DENS_K, DIFF_DENS_K, DIFF_Q1_DENS, DIFF_Q2_DENS, Q1_DENS, Q2_DENS,
-                                             VAR_Q1, VAR_Q1_NONU, VAR_Q2, VAR_Q2_DIAG, VAR_Q2_NONU, Circuit)
+from .quantum_differentiable_circuit import (CONST_GATE_K, CONST_GATE_K_NONU, CONST_Q1, CONST_Q1_NONU, CONST_Q2,
+                                             CONST_Q2_DIAG, CONST_Q2_NONU, DENS_K, DIFF_DENS_K, DIFF_Q1_DENS,
+                                             DIFF_Q2_DENS, Q1_DENS, Q2_DENS, VAR_GATE_K, VAR_GATE_K_NONU, VAR_Q1,
+                                             VAR_Q1_NONU, VAR_Q2, VAR_Q2_DIAG, VAR_Q2_NONU, Circuit)
 
 _Q1 = (CONST_Q1, CONST_Q1_NONU, VAR_Q1, VAR_Q1_NONU)
 _Q2D = (CONST_Q2, VAR_Q2, CONST_Q2_NONU, VAR_Q2_NONU)
 _DIAG = (CONST_Q2_DIAG, VAR_Q2_DIAG)
-_VAR = (VAR_Q2, VAR_Q2_NONU, VAR_Q2_DIAG, VAR_Q1, VAR_Q1_NONU)
+_KGATE = (CONST_GATE_K, VAR_GATE_K, CONST_GATE_K_NONU, VAR_GATE_K_NONU)
+_VAR = (VAR_Q2, VAR_Q2_NONU, VAR_Q2_DIAG, VAR_Q1, VAR_Q1_NONU, VAR_GATE_K, VAR_GATE_K_NONU)
 _NONU = (CONST_Q2_NONU, VAR_Q2_NONU, CONST_Q1_NONU, VAR_Q1_NONU)
 _DENS = (Q2_DENS, Q1_DENS, DIFF_Q2_DENS, DIFF_Q1_DENS, DENS_K, DIFF_DENS_K)
 _SWAP = np.array([0, 2, 1, 3])  # index 2 b_hi + b_lo with the two bits exchanged
@@ -66,13 +70,13 @@ class _XGate:
 
 
 def plan_fusion(program: Sequence[tuple]):
-    """program: [(kind, pos2[, pos1])] -> execution list of ('gate', _XGate) / ('dens', instruction index)."""
+    """program: [(kind, pos2[, pos1])] -> execution list of ('gate', _XGate) / ('dens' | 'kgate', instruction index)."""
     out: List[tuple] = []
     open_gate: Dict[int, _XGate] = {}
     for idx, inst in enumerate(program):
         kind, p2 = inst[0], inst[1]
-        if kind in _DENS:
-            out.append(("dens", idx))
+        if kind in _DENS or kind in _KGATE:
+            out.append(("dens" if kind in _DENS else "kgate", idx))
             open_gate.clear()
             continue
         if kind in _Q1:
@@ -103,7 +107,7 @@ def plan_fusion(program: Sequence[tuple]):
         g.members.append((idx, E_DIAG if diag else E_SAME))
         out.append(("gate", g))
         open_gate[p2] = open_gate[p1] = g
-    return [(t, x) for t, x in out if t == "dens" or x.alive]
+    return [(t, x) for t, x in out if t != "gate" or x.alive]
 
 
 def _fused_kind(g: _XGate, program) -> int:
@@ -197,6 +201,21 @@ class FusedCircuit(Circuit):
         self._kinds.append(kind)
         self._inner = None
 
+    def _add_gate_k(self, positions, variable, non_unitary):
+        if any(p < 0 for p in positions):
+            raise OverflowError("can't convert negative int to unsigned")
+        if not 1 <= len(positions) <= 6:
+            raise ValueError("the number of gate qubits must be in 1..6.")
+        if any(p >= self.qubits_number for p in positions):
+            raise ValueError("pos is out of the bound.")
+        if len(set(positions)) != len(positions):
+            raise ValueError("positions must be different.")
+        kind = (VAR_GATE_K if variable else CONST_GATE_K) if not non_unitary else \
+            (VAR_GATE_K_NONU if variable else CONST_GATE_K_NONU)
+        self._program.append((kind, tuple(positions)))   # a barrier, executed unfused (plan_fusion)
+        self._kinds.append(kind)
+        self._inner = None
+
     def __del__(self):
         pass
 
@@ -241,12 +260,14 @@ class FusedCircuit(Circuit):
         def dens_len(inst):
             k = inst[0]
             return 4 ** len(inst[1]) if k in (DENS_K, DIFF_DENS_K) else 4 if k in (Q1_DENS, DIFF_Q1_DENS) else 16
-        gate_len = lambda k: 16 if k in (CONST_Q2, VAR_Q2, CONST_Q2_NONU, VAR_Q2_NONU) else 4   # noqa: E731
+        def gate_len(inst):
+            k = inst[0]
+            return 4 ** len(inst[1]) if k in _KGATE else 16 if k in (CONST_Q2, VAR_Q2, CONST_Q2_NONU, VAR_Q2_NONU) else 4
         ks, prog = self._kinds, self._program
         diff = (DIFF_Q1_DENS, DIFF_Q2_DENS, DIFF_DENS_K)
         return [len(ks), sum(k not in _DENS and k not in _VAR for k in ks), sum(k in _VAR for k in ks),
                 sum(k in _DENS for k in ks), sum(k in diff for k in ks), sum(dens_len(i) for i in prog if i[0] in _DENS),
-                sum(dens_len(i) for i in prog if i[0] in diff), sum(gate_len(k) for k in ks if k in _VAR)][what]
+                sum(dens_len(i) for i in prog if i[0] in diff), sum(gate_len(i) for i in prog if i[0] in _VAR)][what]
 
     @property
     def fused_gate_count(self) -> int:
@@ -271,10 +292,14 @@ class FusedCircuit(Circuit):
                   VAR_Q2_DIAG: "add_q2_var_gate_diag", CONST_Q1: "add_q1_const_gate",
                   CONST_Q1_NONU: "add_q1_const_gate_nonu", VAR_Q1: "add_q1_var_gate", VAR_Q1_NONU: "add_q1_var_gate_nonu",
                   Q2_DENS: "get_q2_dens_op", Q1_DENS: "get_q1_dens_op", DIFF_Q2_DENS: "get_q2_dens_op_with_grad",
-                  DIFF_Q1_DENS: "get_q1_dens_op_with_grad", DENS_K: "get_dens_op", DIFF_DENS_K: "get_dens_op_with_grad"}
+                  DIFF_Q1_DENS: "get_q1_dens_op_with_grad", DENS_K: "get_dens_op", DIFF_DENS_K: "get_dens_op_with_grad",
+                  CONST_GATE_K: "add_const_gate", VAR_GATE_K: "add_var_gate", CONST_GATE_K_NONU: "add_const_gate_nonu",
+                  VAR_GATE_K_NONU: "add_var_gate_nonu"}
         self._xkinds = []
         for t, x in self._exec:
-            if t == "dens":
+            if t == "kgate":
+                getattr(inner, adders[prog[x][0]])(list(prog[x][1]))
+            elif t == "dens":
                 inst = prog[x]
                 if inst[0] in (DENS_K, DIFF_DENS_K):
                     getattr(inner, adders[inst[0]])(list(inst[1]))
@@ -341,8 +366,17 @@ class FusedCircuit(Circuit):
                     fused[gi] = u[b].diagonal().astype(dt)
                 else:
                     fused[gi] = u[b].reshape(16).astype(dt)
-        cg = [fused[gi] for gi, k in enumerate(self._xkinds) if k not in _VAR]
-        vg = [fused[gi] for gi, k in enumerate(self._xkinds) if k in _VAR]
+        # the inner program's gate lists: fused gates and the (unfused) k-qubit gates, in execution order
+        cg, vg, gi = [], [], 0
+        for t, x in self._exec:
+            if t == "gate":
+                g, k = fused[gi], self._xkinds[gi]
+                gi += 1
+            elif t == "kgate":
+                g, k = lists[self._src[x][0]][self._src[x][1]], self._program[x][0]
+            else:
+                continue
+            (vg if k in _VAR else cg).append(g)
         return cg, vg, keep
 
     def run(self, const_gates, var_gates):
@@ -359,11 +393,16 @@ class FusedCircuit(Circuit):
         dt = np.dtype(getattr(inner, "dtype", np.complex128))
         gfused = inner.backward([np.asarray(g, dtype=dt) for g in grads_wrt_density], cg, vg)
         slot = {}
-        v = 0
-        for gi, k in enumerate(self._xkinds):
-            if k in _VAR:
-                slot[gi] = v; v += 1
         out = [None] * self._n_var
+        v = gi = 0
+        for t, x in self._exec:
+            if t == "gate":
+                if self._xkinds[gi] in _VAR:
+                    slot[gi] = v; v += 1
+                gi += 1
+            elif t == "kgate" and self._program[x][0] in _VAR:
+                out[self._src[x][1]] = np.asarray(gfused[v], dtype=dt)   # gradient of an unfused gate: as it is
+                v += 1
         for sig, gis in self._batches.items():
             one, all_diag, embs, is_var = sig
             if not any(is_var):

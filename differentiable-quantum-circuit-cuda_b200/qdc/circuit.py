@@ -168,6 +168,11 @@ class AutoGradCircuit:
     # densities on 1..6 qubits, positions[0] the most significant bit (Circuit.get_dens_op)
     def get_dens_op(self, positions): self.circuit.get_dens_op(positions)
     def get_dens_op_with_grad(self, positions): self.circuit.get_dens_op_with_grad(positions)
+    # gates on 1..6 qubits, positions[0] the most significant bit (Circuit.add_const_gate)
+    def add_const_gate(self, positions): self.circuit.add_const_gate(positions)
+    def add_var_gate(self, positions): self.circuit.add_var_gate(positions)
+    def add_const_gate_nonu(self, positions): self.circuit.add_const_gate_nonu(positions)
+    def add_var_gate_nonu(self, positions): self.circuit.add_var_gate_nonu(positions)
 
     def build(self) -> Tuple[Callable, Callable]:
         """Returns (simple_run, autodiff_run), src/qdc/circuit.py:160-202.

@@ -24,9 +24,10 @@ import numpy as np
 
 from .._ffi import Lib, ProfileEntry, QdcError, Stats, default_precision, get_lib
 
-# enum Instruction, src/circuit.rs:53-68, then the densities on 3..6 qubits (include/qdc_circuit.h)
+# enum Instruction, src/circuit.rs:53-68, then the densities and the gates on 3..6 qubits (include/qdc_circuit.h)
 (CONST_Q2, VAR_Q2, CONST_Q2_NONU, VAR_Q2_NONU, CONST_Q2_DIAG, VAR_Q2_DIAG, CONST_Q1, CONST_Q1_NONU, VAR_Q1,
- VAR_Q1_NONU, Q2_DENS, Q1_DENS, DIFF_Q2_DENS, DIFF_Q1_DENS, DENS_K, DIFF_DENS_K) = range(16)
+ VAR_Q1_NONU, Q2_DENS, Q1_DENS, DIFF_Q2_DENS, DIFF_Q1_DENS, DENS_K, DIFF_DENS_K, CONST_GATE_K, VAR_GATE_K,
+ CONST_GATE_K_NONU, VAR_GATE_K_NONU) = range(20)
 
 (N_INSTRUCTIONS, N_CONST_GATES, N_VAR_GATES, N_DENSITIES, N_DIFF_DENSITIES, RUN_OUT_LEN, FORWARD_OUT_LEN,
  BACKWARD_OUT_LEN) = range(8)
@@ -40,7 +41,7 @@ class Circuit:
         self._lib.call("qdc_circuit_new", C.byref(h), self.qubits_number)
         self._h = h
         self._kinds: List[int] = []
-        self._dims: List[int] = []   # side of every instruction's density output (0: a gate)
+        self._dims: List[int] = []   # side of every instruction's density output or k-qubit gate matrix (else 0)
 
     def __del__(self):
         try:
@@ -77,6 +78,15 @@ class Circuit:
         self._kinds.append(DIFF_DENS_K if with_grad else DENS_K)
         self._dims.append(1 << pos.size)
 
+    def _add_gate_k(self, positions: List[int], variable: bool, non_unitary: bool):
+        if any(p < 0 for p in positions):
+            raise OverflowError("can't convert negative int to unsigned")
+        pos = np.array(positions, dtype=np.uintp)
+        self._lib.call("qdc_circuit_add_gate", self._h, pos.ctypes.data, pos.size, int(variable), int(non_unitary))
+        self._kinds.append((VAR_GATE_K if variable else CONST_GATE_K) if not non_unitary
+                           else (VAR_GATE_K_NONU if variable else CONST_GATE_K_NONU))
+        self._dims.append(1 << pos.size)
+
     def add_q2_const_gate(self, pos2: int, pos1: int): self._add(CONST_Q2, pos2, pos1)
     def add_q2_const_gate_diag(self, pos2: int, pos1: int): self._add(CONST_Q2_DIAG, pos2, pos1)
     def add_q2_const_gate_nonu(self, pos2: int, pos1: int): self._add(CONST_Q2_NONU, pos2, pos1)
@@ -101,6 +111,35 @@ class Circuit:
     def get_dens_op_with_grad(self, positions: Sequence[int]):
         """`get_dens_op` with gradient: forward returns it, backward takes its (2^k, 2^k) cotangent."""
         self._add_dens(positions, True)
+
+    def add_const_gate(self, positions: Sequence[int]):
+        """Gate on the qubits `positions` = [p_{k-1}, ..., p_0] (1 <= k <= 6, distinct, any order), positions[0] the
+        most significant bit of its row and column index: psi'[r, rest] = sum_c U[r, c] psi[c, rest].  U is taken
+        flat (4^k entries, row-major) from the constant gate list.  k = 1 and 2 are add_q1_const_gate(p) and
+        add_q2_const_gate(p2, p1)."""
+        self._add_gate(positions, False, False)
+
+    def add_var_gate(self, positions: Sequence[int]):
+        """`add_const_gate` from the variable gate list: backward returns its (4^k-entry) gradient."""
+        self._add_gate(positions, True, False)
+
+    def add_const_gate_nonu(self, positions: Sequence[int]):
+        """`add_const_gate` for a non-unitary U (the reverse pass un-computes with its inverse)."""
+        self._add_gate(positions, False, True)
+
+    def add_var_gate_nonu(self, positions: Sequence[int]):
+        """`add_var_gate` for a non-unitary U."""
+        self._add_gate(positions, True, True)
+
+    def _add_gate(self, positions, variable: bool, non_unitary: bool):
+        pos = [int(p) for p in positions]
+        if len(pos) == 1:
+            getattr(self, "add_q1_%s_gate%s" % ("var" if variable else "const", "_nonu" if non_unitary else ""))(pos[0])
+        elif len(pos) == 2:
+            getattr(self, "add_q2_%s_gate%s" % ("var" if variable else "const", "_nonu" if non_unitary else ""))(
+                pos[0], pos[1])
+        else:
+            self._add_gate_k(pos, variable, non_unitary)
 
     def _add_dens(self, positions, with_grad: bool):
         pos = [int(p) for p in positions]
@@ -167,11 +206,13 @@ class Circuit:
                        cf.ctypes.data, cl.ctypes.data, cl.size, vf.ctypes.data, vl.ctypes.data, vl.size,
                        out.ctypes.data, cap, C.byref(n_out))
         res, o = [], 0
-        for k in self._kinds:
+        for k, m in zip(self._kinds, self._dims):
             if k in (VAR_Q2, VAR_Q2_NONU):
                 res.append(out[o:o + 16].copy()); o += 16
             elif k in (VAR_Q2_DIAG, VAR_Q1, VAR_Q1_NONU):
                 res.append(out[o:o + 4].copy()); o += 4
+            elif k in (VAR_GATE_K, VAR_GATE_K_NONU):
+                res.append(out[o:o + m * m].copy()); o += m * m
         assert o == n_out.value
         return res
 

@@ -31,13 +31,15 @@ extern "C" {
 typedef struct qdc_circuit qdc_circuit;
 
 /* Instruction kinds == `enum Instruction`, src/circuit.rs:53-68 (same order),
- * then the densities on 3..6 qubits, which only qdc_circuit_add_dens adds. */
+ * then the densities on 3..6 qubits, which only qdc_circuit_add_dens adds,
+ * then the gates on 3..6 qubits, which only qdc_circuit_add_gate adds. */
 enum qdc_kind {
   QDC_CONST_Q2 = 0, QDC_VAR_Q2 = 1, QDC_CONST_Q2_NONU = 2, QDC_VAR_Q2_NONU = 3,
   QDC_CONST_Q2_DIAG = 4, QDC_VAR_Q2_DIAG = 5,
   QDC_CONST_Q1 = 6, QDC_CONST_Q1_NONU = 7, QDC_VAR_Q1 = 8, QDC_VAR_Q1_NONU = 9,
   QDC_Q2_DENS = 10, QDC_Q1_DENS = 11, QDC_DIFF_Q2_DENS = 12, QDC_DIFF_Q1_DENS = 13,
-  QDC_DENS_K = 14, QDC_DIFF_DENS_K = 15
+  QDC_DENS_K = 14, QDC_DIFF_DENS_K = 15,
+  QDC_CONST_GATE_K = 16, QDC_VAR_GATE_K = 17, QDC_CONST_GATE_K_NONU = 18, QDC_VAR_GATE_K_NONU = 19
 };
 
 /* qdc_circuit_count selectors */
@@ -73,7 +75,8 @@ const char* qdc_circuit_free(qdc_circuit* c);
 /* Circuit::set_state_from_vector, src/circuit.rs:104-106 */
 const char* qdc_circuit_set_state_from_host(qdc_circuit* c, const qdc_complex* host_state, size_t len);
 /* The 14 builder methods, src/circuit.rs:108-162.  pos1 is ignored for q1 kinds.
- * QDC_DENS_K / QDC_DIFF_DENS_K are refused here (they need qdc_circuit_add_dens). */
+ * QDC_DENS_K / QDC_DIFF_DENS_K are refused here (they need qdc_circuit_add_dens), and so are
+ * QDC_*_GATE_K* (they need qdc_circuit_add_gate). */
 const char* qdc_circuit_add(qdc_circuit* c, int kind, size_t pos2, size_t pos1);
 /* Reduced density matrix on k = 1..6 distinct qubits positions[0..k-1] (positions[0] is the most
  * significant bit of the row and column index), with gradient if `with_grad`:
@@ -82,6 +85,19 @@ const char* qdc_circuit_add(qdc_circuit* c, int kind, size_t pos2, size_t pos1);
  * k >= 3 adds QDC_(DIFF_)DENS_K.  Like every density it is a barrier; run / forward return it in program
  * order and backward takes its (conjugated) 4^k-entry cotangent in program order. */
 const char* qdc_circuit_add_dens(qdc_circuit* c, const size_t* positions, size_t k, int with_grad);
+/* Gate on k = 1..6 distinct qubits positions[0..k-1] (positions[0] is the most significant bit of the
+ * row and column index), constant or `variable` (with gradient), unitary or `non_unitary`:
+ *   psi'[r, rest] = sum_c U[r, c] psi[c, rest],   U: 2^k x 2^k, row-major, 4^k entries, taken in
+ *   program order from the const / var gate lists like every other gate.
+ * The reverse pass un-computes with U^dagger (U^-1 for non_unitary, Gauss-Jordan in double precision;
+ * a singular pivot fails with "U(i, i) is zero."), returns G[r, c] = sum_rest bwd[r, rest] fwd[c, rest]
+ * (4^k entries, no conjugation, like the two-qubit gradient) and pulls the adjoint back with U^T.
+ * A variable gate after the last differentiable density has a zero gradient, like every gate kind.
+ * k = 1 and 2 add QDC_{CONST,VAR}_Q1[_NONU](positions[0]) and QDC_{CONST,VAR}_Q2[_NONU](positions[0],
+ * positions[1]); k >= 3 adds QDC_{CONST,VAR}_GATE_K[_NONU], a barrier like a density: the executor moves
+ * no instruction across it. */
+const char* qdc_circuit_add_gate(qdc_circuit* c, const size_t* positions, size_t k, int variable,
+                                 int non_unitary);
 size_t qdc_circuit_count(const qdc_circuit* c, int what);
 
 /* Circuit::run, src/circuit.rs:164-212 (all densities, program order). */
