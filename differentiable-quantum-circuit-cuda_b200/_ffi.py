@@ -56,6 +56,7 @@ _CIRCUIT_SIGNATURES = {
     "qdc_circuit_add": (_err, [C.c_void_p, C.c_int, _sz, _sz]),
     "qdc_circuit_add_dens": (_err, [C.c_void_p, C.c_void_p, _sz, C.c_int]),
     "qdc_circuit_add_gate": (_err, [C.c_void_p, C.c_void_p, _sz, C.c_int, C.c_int]),
+    "qdc_circuit_add_gate_diag": (_err, [C.c_void_p, C.c_void_p, _sz, C.c_int, C.c_int]),
     "qdc_circuit_count": (_sz, [C.c_void_p, C.c_int]),
     "qdc_circuit_run": (_err, [C.c_void_p, c_cplx_p, _u32p, _sz, c_cplx_p, _u32p, _sz, c_cplx_p, _sz,
                                C.POINTER(_sz)]),

@@ -16,6 +16,7 @@
 #include <string>
 #include <vector>
 
+#include "diag_k_host.hpp"
 #include "engine.cuh"
 #include "nccl_dyn.hpp"
 #include "scheduler.hpp"
@@ -28,24 +29,27 @@ enum Kind {
   K_CONST_Q1, K_CONST_Q1_NONU, K_VAR_Q1, K_VAR_Q1_NONU,
   K_Q2_DENS, K_Q1_DENS, K_DIFF_Q2_DENS, K_DIFF_Q1_DENS,
   K_DENS_K, K_DIFF_DENS_K,  // densities on 3..6 qubits (add_dens; dens_k_kernels.cuh)
-  K_CONST_GATE_K, K_VAR_GATE_K, K_CONST_GATE_K_NONU, K_VAR_GATE_K_NONU   // gates on 3..6 qubits (add_gate; gate_k_kernels.cuh)
+  K_CONST_GATE_K, K_VAR_GATE_K, K_CONST_GATE_K_NONU, K_VAR_GATE_K_NONU,  // gates on 3..6 qubits (add_gate; gate_k_kernels.cuh)
+  K_CONST_DIAG_K, K_VAR_DIAG_K, K_CONST_DIAG_K_NONU, K_VAR_DIAG_K_NONU   // diagonal gates on 1..6 qubits (add_gate_diag;
+                                                                         // diag_k_kernels.cuh)
 };
 
 // one- and two-qubit gates (the k-qubit gates are kind_is_k_gate)
 static inline bool kind_is_gate(int k) { return k <= K_VAR_Q1_NONU; }
 static inline bool kind_is_var(int k) {
   return k == K_VAR_Q2 || k == K_VAR_Q2_NONU || k == K_VAR_Q2_DIAG || k == K_VAR_Q1 || k == K_VAR_Q1_NONU ||
-         k == K_VAR_GATE_K || k == K_VAR_GATE_K_NONU;
+         k == K_VAR_GATE_K || k == K_VAR_GATE_K_NONU || k == K_VAR_DIAG_K || k == K_VAR_DIAG_K_NONU;
 }
 static inline bool kind_is_nonu(int k) {
   return k == K_CONST_Q2_NONU || k == K_VAR_Q2_NONU || k == K_CONST_Q1_NONU || k == K_VAR_Q1_NONU ||
-         k == K_CONST_GATE_K_NONU || k == K_VAR_GATE_K_NONU;
+         k == K_CONST_GATE_K_NONU || k == K_VAR_GATE_K_NONU || k == K_CONST_DIAG_K_NONU || k == K_VAR_DIAG_K_NONU;
 }
 static inline bool kind_is_diag(int k) { return k == K_CONST_Q2_DIAG || k == K_VAR_Q2_DIAG; }
 static inline bool kind_is_q1(int k) { return k >= K_CONST_Q1 && k <= K_VAR_Q1_NONU; }
 static inline bool kind_is_q2dense(int k) { return k <= K_VAR_Q2_NONU; }
 static inline bool kind_is_dens(int k) { return k >= K_Q2_DENS && k <= K_DIFF_DENS_K; }
 static inline bool kind_is_k_gate(int k) { return k >= K_CONST_GATE_K && k <= K_VAR_GATE_K_NONU; }
+static inline bool kind_is_diag_k(int k) { return k >= K_CONST_DIAG_K && k <= K_VAR_DIAG_K_NONU; }
 static inline bool kind_is_diff_dens(int k) { return k == K_DIFF_Q2_DENS || k == K_DIFF_Q1_DENS || k == K_DIFF_DENS_K; }
 static inline bool kind_is_k_dens(int k) { return k == K_DENS_K || k == K_DIFF_DENS_K; }
 static inline bool kind_is_q1_dens(int k) { return k == K_Q1_DENS || k == K_DIFF_Q1_DENS; }
@@ -55,7 +59,7 @@ static inline int kind_dens_len(int k) { return kind_is_q1_dens(k) ? 4 : 16; }
 struct Inst {
   int kind;
   int pos2, pos1;  // q1 kinds use pos2 only
-  int nk = 0;      // k-qubit densities and gates: the qubits kpos[0..nk-1], most significant first (pos2 = pos1 = -1)
+  int nk = 0;      // k-qubit densities and gates (dense, diagonal): the qubits kpos[0..nk-1], most significant first (pos2 = pos1 = -1)
   int kpos[6] = {-1, -1, -1, -1, -1, -1};
 };
 
@@ -66,6 +70,7 @@ static inline size_t dens_len(const Inst& in) {
 
 // complex entries of a gate's matrix / gradient
 static inline size_t gate_len(const Inst& in) {
+  if (kind_is_diag_k(in.kind)) return (size_t)1 << in.nk;
   return kind_is_k_gate(in.kind) ? (size_t)1 << (2 * in.nk) : (size_t)kind_gate_len(in.kind);
 }
 
@@ -76,6 +81,7 @@ struct Stats {
 struct DensGroup;
 struct TileDensParams;
 struct DensKParams;
+struct DiagKPos;
 struct TcState;
 struct TcPass;
 
@@ -90,11 +96,12 @@ struct GateList {
 enum ProfCat {
   CAT_FWD_Q1 = 0, CAT_FWD_Q2, CAT_FWD_DIAG, CAT_DENSITY, CAT_SEED, CAT_UNCOMPUTE, CAT_REV_Q1, CAT_REV_Q2,
   CAT_REV_DIAG, CAT_REV_CONST, CAT_TILE_FWD, CAT_TILE_BWD, CAT_EXCHANGE, CAT_TC_FWD, CAT_TC_BWD, CAT_GATE_K_FWD,
-  CAT_GATE_K_REV, CAT_COUNT
+  CAT_GATE_K_REV, CAT_DIAG_K_FWD, CAT_DIAG_K_REV, CAT_COUNT
 };
 static const char* const kProfCatNames[CAT_COUNT] = {
     "fwd_q1", "fwd_q2", "fwd_diag", "density", "seed", "uncompute", "rev_q1", "rev_q2",
-    "rev_diag", "rev_const", "tile_fwd", "tile_bwd", "exchange", "tc_fwd", "tc_bwd", "gate_k_fwd", "gate_k_rev"};
+    "rev_diag", "rev_const", "tile_fwd", "tile_bwd", "exchange", "tc_fwd", "tc_bwd", "gate_k_fwd", "gate_k_rev",
+    "diag_k_fwd", "diag_k_rev"};
 
 struct ProfEntry {
   uint64_t launches = 0;
@@ -308,8 +315,9 @@ class Circuit {
   size_t d_kmat_cap_ = 0;
   std::vector<cplx_t> h_kmat_;
   std::vector<size_t> kmat_ofs_;
-  // k-qubit gates: their device forms share the cotangents' region and copy (at gmat_ofs_[instruction]); the
-  // gradients of the variable ones follow the 32-double slots in d_res_ (at kgofs_[instruction], in doubles)
+  // k-qubit gates, dense and diagonal: their device forms share the cotangents' region and copy (at
+  // gmat_ofs_[instruction]); the gradients of the variable ones follow the 32-double slots in d_res_ (at
+  // kgofs_[instruction], in doubles)
   std::vector<size_t> gmat_ofs_, kgofs_;
   cudaStream_t stream_ = 0;
   Stats stats_;
@@ -492,6 +500,7 @@ class Circuit {
   const char* add(int kind, size_t pos2, size_t pos1) {
     if (kind_is_k_dens(kind)) return qdc_errf("kind %d carries its qubits through qdc_circuit_add_dens.", kind);
     if (kind_is_k_gate(kind)) return qdc_errf("kind %d carries its qubits through qdc_circuit_add_gate.", kind);
+    if (kind_is_diag_k(kind)) return qdc_errf("kind %d carries its qubits through qdc_circuit_add_gate_diag.", kind);
     if (kind < 0 || kind > K_DIFF_Q1_DENS) return qdc_errf("Unknown instruction kind %d.", kind);
     const bool one = kind_is_q1(kind) || kind_is_q1_dens(kind);
     if (one) {
@@ -549,11 +558,30 @@ class Circuit {
     return nullptr;
   }
 
+  // Diagonal gate on k = 1..6 qubits, positions[0] the most significant bit of its index j; a unitary one on
+  // k = 2 adds the two-qubit diagonal kinds.
+  const char* add_gate_diag(const size_t* positions, size_t k, bool variable, bool non_unitary) {
+    if (k < 1 || k > 6) return qdc_errf("the number of gate qubits must be in 1..6, got %zu.", k);
+    if (k == 2 && !non_unitary) return add(variable ? K_VAR_Q2_DIAG : K_CONST_Q2_DIAG, positions[0], positions[1]);
+    Inst in{variable ? (non_unitary ? K_VAR_DIAG_K_NONU : K_VAR_DIAG_K)
+                     : (non_unitary ? K_CONST_DIAG_K_NONU : K_CONST_DIAG_K), -1, -1};
+    for (size_t j = 0; j < k; j++) {
+      if (positions[j] >= (size_t)n_) return qdc_errf("pos is out of the bound.");
+      for (size_t i = 0; i < j; i++)
+        if (positions[i] == positions[j]) return qdc_errf("positions must be different.");
+      in.kpos[j] = (int)positions[j];
+    }
+    in.nk = (int)k;
+    insts_.push_back(in);
+    forward_valid_ = false;
+    return nullptr;
+  }
+
   size_t count(int what) const {
     size_t c = 0;
     for (const Inst& in : insts_) {
       const int k = in.kind;
-      const bool gate = kind_is_gate(k) || kind_is_k_gate(k);
+      const bool gate = kind_is_gate(k) || kind_is_k_gate(k) || kind_is_diag_k(k);
       switch (what) {
         case 0: c++; break;
         case 1: c += gate && !kind_is_var(k); break;
@@ -576,7 +604,7 @@ class Circuit {
     size_t ci = 0, vi = 0, coff = 0, voff = 0;
     for (size_t i = 0; i < insts_.size(); i++) {
       const int k = insts_[i].kind;
-      if (!kind_is_gate(k) && !kind_is_k_gate(k)) continue;
+      if (!kind_is_gate(k) && !kind_is_k_gate(k) && !kind_is_diag_k(k)) continue;
       const bool var = kind_is_var(k);
       const GateList& gl = var ? vg : cg;
       size_t& idx = var ? vi : ci;
@@ -739,6 +767,7 @@ class Circuit {
     if (kind_is_diag(k)) return 2;
     if (kind_is_k_dens(k)) return 5;
     if (kind_is_k_gate(k)) return 6;
+    if (kind_is_diag_k(k)) return 7;
     return kind_is_q1_dens(k) ? 3 : 4;
   }
 
@@ -1094,14 +1123,14 @@ class Circuit {
       d_kres_cap_ = nkres;
     }
     h_kres_.resize(nkres);
-    h_kmat_.clear();
-    QDC_TRY(add_gate_k_forms(gp, false));
-    QDC_TRY(upload_kmat());
     forward_valid_ = false;
-    build_plan(all_dens);
+    build_plan(all_dens);   // (the diagonal k-qubit gates' forms depend on where the plan runs them)
     if (!plan_.ok)
       return qdc_errf("the program cannot be scheduled on %d local qubits per rank (an instruction never has all "
                       "its qubits local).", n_loc_);
+    h_kmat_.clear();
+    QDC_TRY(add_gate_k_forms(gp, false));
+    QDC_TRY(upload_kmat());
     QDC_TRY(reset_state());
     if (nslots) QDC_CUDA(cudaMemsetAsync(d_res_, 0, nslots * 32 * sizeof(double), stream_));
 #ifndef QDC_F64
@@ -1220,6 +1249,9 @@ class Circuit {
         case qdc::ST_GATE_K:
           QDC_TRY(gate_k_apply(st, state_, d_kmat_ + gmat_ofs_[st.inst], CAT_GATE_K_FWD));
           break;
+        case qdc::ST_DIAG_K:
+          QDC_TRY(diag_k_apply(st, state_, d_kmat_ + gmat_ofs_[st.inst], CAT_DIAG_K_FWD));
+          break;
       }
     }
     return nullptr;
@@ -1247,7 +1279,8 @@ class Circuit {
     return nullptr;
   }
 
-  // Appends the device forms of every k-qubit gate (gate_k_forms) to h_kmat_, at gmat_ofs_[instruction].
+  // Appends the device forms of every k-qubit gate (gate_k_forms, diag_k_forms) to h_kmat_, at
+  // gmat_ofs_[instruction].
   const char* add_gate_k_forms(const std::vector<const cplx_t*>& gp, bool reverse) {
     gmat_ofs_.assign(insts_.size(), 0);
     for (size_t i = 0; i < insts_.size(); i++) {
@@ -1255,6 +1288,11 @@ class Circuit {
       if (!kind_is_k_gate(in.kind)) continue;
       gmat_ofs_[i] = h_kmat_.size();
       QDC_TRY(gate_k_forms(gp[i], in.nk, kind_is_nonu(in.kind), reverse, &h_kmat_));
+    }
+    for (const qdc::Step& st : plan_.steps) {   // diagonal ones: folded over the rank bits of their plan step
+      if (st.type != qdc::ST_DIAG_K) continue;
+      gmat_ofs_[st.inst] = h_kmat_.size();
+      QDC_TRY(diag_k_forms(gp[st.inst], insts_[st.inst], st.pk, reverse, &h_kmat_));
     }
     return nullptr;
   }
@@ -1325,7 +1363,7 @@ class Circuit {
     size_t ndbl = nvar * 32;
     kgofs_.assign(insts_.size(), 0);
     for (size_t i = 0; i < insts_.size(); i++) {
-      if (!kind_is_k_gate(insts_[i].kind) || !kind_is_var(insts_[i].kind)) continue;
+      if (!(kind_is_k_gate(insts_[i].kind) || kind_is_diag_k(insts_[i].kind)) || !kind_is_var(insts_[i].kind)) continue;
       kgofs_[i] = ndbl;
       ndbl += 2 * gate_len(insts_[i]);
     }
@@ -1356,6 +1394,17 @@ class Circuit {
           out[o + j].y = (real_t)h[2 * j + 1];
         }
         o += len;
+        continue;
+      }
+      if (kind_is_diag_k(in.kind) && kind_is_var(in.kind)) {
+        // the kernel's 2^k_loc entries -> the gate's 2^k entries at this rank's bits
+        std::vector<zc> g;
+        qdc::diag_scatter(qdc::diag_fold_split(exec_pk(i), in.nk, n_loc_, rank_), in.nk, &h_res_[kgofs_[i]], &g);
+        for (size_t j = 0; j < g.size(); j++) {
+          out[o + j].x = (real_t)g[j].real();
+          out[o + j].y = (real_t)g[j].imag();
+        }
+        o += g.size();
         continue;
       }
       if (vslot[i] < 0) continue;
@@ -1457,6 +1506,15 @@ class Circuit {
           if (!live) QDC_TRY(gate_k_apply(st, state_, inv, CAT_GATE_K_REV));
           else QDC_TRY(gate_k_reverse(st, inv, inv + ((size_t)1 << (2 * st.nk)),
                                       kind_is_var(k) ? d_res_ + kgofs_[st.inst] : nullptr));
+          break;
+        }
+        case qdc::ST_DIAG_K: {
+          // forms: the un-compute form, then d, 2^k_loc entries each; no adjoint yet: un-compute only
+          const cplx_t* inv = d_kmat_ + gmat_ofs_[st.inst];
+          const int k = insts_[st.inst].kind;
+          const size_t len = (size_t)1 << qdc::diag_fold_split(st.pk, st.nk, n_loc_, rank_).k_loc;
+          if (!live) QDC_TRY(diag_k_apply(st, state_, inv, CAT_DIAG_K_REV));
+          else QDC_TRY(diag_k_reverse(st, inv, inv + len, kind_is_var(k) ? d_res_ + kgofs_[st.inst] : nullptr));
           break;
         }
         case qdc::ST_TILE:
@@ -1565,6 +1623,20 @@ class Circuit {
                                                   double* gdst);
   const char* gate_k_apply(const qdc::Step& st, cplx_t* buf, const cplx_t* At, int cat);
   const char* gate_k_reverse(const qdc::Step& st, const cplx_t* At, const cplx_t* Bt, double* gdst);
+  // diagonal k-qubit gates (diag_k_kernels.cuh)
+  const char* diag_k_forms(const cplx_t* d, const Inst& in, const int* pk, bool reverse, std::vector<cplx_t>* h);
+  const char* launch_diag_k(cplx_t* buf, const cplx_t* form, const DiagKPos& p);
+  const char* launch_diag_k_rev_whole(const DiagKPos& p, const cplx_t* A, const cplx_t* B, double* gdst);
+  template <int NI> const char* launch_diag_k_rev(const DensKParams& dp, const DiagKPos& p, const cplx_t* A,
+                                                  const cplx_t* B, double* gdst);
+  const char* diag_k_apply(const qdc::Step& st, cplx_t* buf, const cplx_t* form, int cat);
+  const char* diag_k_reverse(const qdc::Step& st, const cplx_t* A, const cplx_t* B, double* gdst);
+  // physical positions of the plan step of diagonal k-qubit instruction i
+  const int* exec_pk(size_t i) const {
+    for (const qdc::Step& st : plan_.steps)
+      if (st.type == qdc::ST_DIAG_K && st.inst == (int)i) return st.pk;
+    return insts_[i].kpos;
+  }
   std::vector<char> diag_hilo_;  // diagonal gradient of this instruction came back in (hi,lo) order
   double* tile_partials_ = nullptr;
   size_t tile_partials_cap_ = 0;

@@ -9,6 +9,7 @@
 #include "tile_dens_kernels.cuh"
 #include "dens_k_kernels.cuh"
 #include "gate_k_kernels.cuh"
+#include "diag_k_kernels.cuh"
 #include "tc_exec.cuh"
 
 struct qdc_circuit {
@@ -24,7 +25,7 @@ QDC_EXPORT const char* qdc_precision(void) {
 #endif
 }
 
-QDC_EXPORT int qdc_abi_version(void) { return 4; }
+QDC_EXPORT int qdc_abi_version(void) { return 5; }
 
 QDC_EXPORT const char* qdc_circuit_new(qdc_circuit** out, size_t qubits_number) {
   if (qubits_number < 1 || qubits_number > 40) return qdc_errf("qubits_number out of range.");
@@ -83,6 +84,11 @@ QDC_EXPORT const char* qdc_circuit_add_dens(qdc_circuit* c, const size_t* positi
 QDC_EXPORT const char* qdc_circuit_add_gate(qdc_circuit* c, const size_t* positions, size_t k, int variable,
                                             int non_unitary) {
   return c->impl.add_gate(positions, k, variable != 0, non_unitary != 0);
+}
+
+QDC_EXPORT const char* qdc_circuit_add_gate_diag(qdc_circuit* c, const size_t* positions, size_t k, int variable,
+                                                 int non_unitary) {
+  return c->impl.add_gate_diag(positions, k, variable != 0, non_unitary != 0);
 }
 
 QDC_EXPORT size_t qdc_circuit_count(const qdc_circuit* c, int what) { return c->impl.count(what); }

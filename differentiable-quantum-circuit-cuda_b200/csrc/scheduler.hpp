@@ -13,6 +13,9 @@
 //    non-unitary directions change).  A k-qubit density (kind class 5) needs
 //    all its k qubits local at once.  So does a k-qubit gate (class 6, step
 //    ST_GATE_K), which is a full barrier too: nothing is reordered across it.
+//    A diagonal k-qubit gate (class 7, step ST_DIAG_K) is a full barrier as
+//    well, but like the two-qubit diagonal it needs no local qubit: its rank
+//    bits only select entries, so it never causes a remap.
 //
 // Sharding: with 2^g ranks the top g PHYSICAL bit positions are the rank
 // index ("global").  A logical->physical qubit map is maintained; dense gates
@@ -33,7 +36,7 @@
 
 namespace qdc {
 
-enum StepType : int { ST_GATE = 0, ST_DENS = 1, ST_SWAP = 2, ST_TILE = 3, ST_GATE_K = 4 };
+enum StepType : int { ST_GATE = 0, ST_DENS = 1, ST_SWAP = 2, ST_TILE = 3, ST_GATE_K = 4, ST_DIAG_K = 5 };
 
 struct Step {
   int type = ST_GATE;
@@ -43,12 +46,13 @@ struct Step {
   int first = 0, count = 0;  // TILE: range in Plan::tile_steps
   int tb_first = 0, tb_count = 0;  // TILE: range in Plan::tile_bits (sorted physical positions)
   int grp_first = 0, grp_count = 0;  // TILE: range in Plan::groups (register-block groups)
-  int nk = 0, pk[6] = {-1, -1, -1, -1, -1, -1};  // k-qubit DENS / GATE_K (p2 = p1 = -1): physical positions, most significant first
+  int nk = 0, pk[6] = {-1, -1, -1, -1, -1, -1};  // k-qubit DENS / GATE_K / DIAG_K (p2 = p1 = -1): physical positions, most significant first
 };
 
-// Steps nothing may be moved across: densities and k-qubit gates.  (A k-qubit gate has p2 = p1 = -1, so it marks
-// no position dirty: treated as an ordinary deferred step, later gates on its qubits could overtake it.)
-inline bool is_wall(const Step& st) { return st.type == ST_DENS || st.type == ST_GATE_K; }
+// Steps nothing may be moved across: densities and k-qubit gates, dense or diagonal.  (A k-qubit gate has
+// p2 = p1 = -1, so it marks no position dirty: treated as an ordinary deferred step, later gates on its qubits could
+// overtake it.)
+inline bool is_wall(const Step& st) { return st.type == ST_DENS || st.type == ST_GATE_K || st.type == ST_DIAG_K; }
 
 // A register-block group inside a tile pass: `count` consecutive tile gates
 // (starting at Plan::tile_steps[first]) that all act within <= 4 positions.
@@ -69,10 +73,10 @@ struct Plan {
 
 struct SchedInst {
   int kind_class;  // 0: dense q1, 1: dense q2, 2: diagonal q2, 3: density q1, 4: density q2, 5: density on nq qubits,
-                   // 6: gate on nq qubits
-  int q2, q1;      // logical qubits (q1 = -1 for one-qubit instructions; both -1 for classes 5 and 6)
+                   // 6: gate on nq qubits, 7: diagonal gate on nq qubits
+  int q2, q1;      // logical qubits (q1 = -1 for one-qubit instructions; both -1 for classes 5, 6 and 7)
   bool skip;       // densities that this sweep does not evaluate
-  int nq = 0;      // classes 5 and 6: the logical qubits qk[0..nq-1], most significant first
+  int nq = 0;      // classes 5, 6 and 7: the logical qubits qk[0..nq-1], most significant first
   int qk[6] = {-1, -1, -1, -1, -1, -1};
 };
 
@@ -136,7 +140,7 @@ class Scheduler {
   std::vector<bool> done_;
   std::vector<int> map_;  // logical -> physical
 
-  bool is_barrier(const SchedInst& s) const { return s.kind_class >= 3; }   // densities and k-qubit gates
+  bool is_barrier(const SchedInst& s) const { return s.kind_class >= 3; }   // densities and k-qubit gates (dense, diagonal)
   bool local(int q) const { return map_[q] < o_.n_loc; }
 
   // One sweep in program order: every instruction whose predecessors (on its
@@ -152,9 +156,10 @@ class Scheduler {
         // barrier: runs only if everything before it is done
         if (any_blocked) break;
         bool ok = s.nq > 0 || (local(s.q2) && (s.q1 < 0 || local(s.q1)));
-        for (int j = 0; j < s.nq; j++) ok = ok && local(s.qk[j]);
+        if (s.kind_class != 7)   // a diagonal k-qubit gate runs wherever its qubits are
+          for (int j = 0; j < s.nq; j++) ok = ok && local(s.qk[j]);
         if (!ok) break;
-        ready.push_back(make_step(i, s.kind_class == 6 ? ST_GATE_K : ST_DENS));
+        ready.push_back(make_step(i, s.kind_class == 7 ? ST_DIAG_K : s.kind_class == 6 ? ST_GATE_K : ST_DENS));
         done_[i] = true;
         continue;
       }
@@ -458,7 +463,7 @@ class Scheduler {
     const int N = (int)in_.size();
     std::vector<int> nu(o_.n, N + 1);
     for (int i = N - 1; i >= 0; i--) {
-      if (done_[i]) continue;
+      if (done_[i] || in_[i].kind_class == 7) continue;   // a diagonal k-qubit gate needs none of its qubits local
       // (the qubits of a k-qubit density or gate share one next use: a remap for it never evicts another of them,
       // the victims must be strictly less urgent)
       for (int j = 0; j < in_[i].nq; j++) nu[in_[i].qk[j]] = i;

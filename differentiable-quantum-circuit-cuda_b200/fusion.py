@@ -38,16 +38,20 @@ from typing import Callable, Dict, List, Sequence
 
 import numpy as np
 
-from .quantum_differentiable_circuit import (CONST_GATE_K, CONST_GATE_K_NONU, CONST_Q1, CONST_Q1_NONU, CONST_Q2,
-                                             CONST_Q2_DIAG, CONST_Q2_NONU, DENS_K, DIFF_DENS_K, DIFF_Q1_DENS,
-                                             DIFF_Q2_DENS, Q1_DENS, Q2_DENS, VAR_GATE_K, VAR_GATE_K_NONU, VAR_Q1,
-                                             VAR_Q1_NONU, VAR_Q2, VAR_Q2_DIAG, VAR_Q2_NONU, Circuit)
+from .quantum_differentiable_circuit import (CONST_GATE_K, CONST_GATE_K_DIAG, CONST_GATE_K_DIAG_NONU,
+                                             CONST_GATE_K_NONU, CONST_Q1, CONST_Q1_NONU, CONST_Q2, CONST_Q2_DIAG,
+                                             CONST_Q2_NONU, DENS_K, DIFF_DENS_K, DIFF_Q1_DENS, DIFF_Q2_DENS, Q1_DENS,
+                                             Q2_DENS, VAR_GATE_K, VAR_GATE_K_DIAG, VAR_GATE_K_DIAG_NONU,
+                                             VAR_GATE_K_NONU, VAR_Q1, VAR_Q1_NONU, VAR_Q2, VAR_Q2_DIAG, VAR_Q2_NONU,
+                                             Circuit)
 
 _Q1 = (CONST_Q1, CONST_Q1_NONU, VAR_Q1, VAR_Q1_NONU)
 _Q2D = (CONST_Q2, VAR_Q2, CONST_Q2_NONU, VAR_Q2_NONU)
 _DIAG = (CONST_Q2_DIAG, VAR_Q2_DIAG)
-_KGATE = (CONST_GATE_K, VAR_GATE_K, CONST_GATE_K_NONU, VAR_GATE_K_NONU)
-_VAR = (VAR_Q2, VAR_Q2_NONU, VAR_Q2_DIAG, VAR_Q1, VAR_Q1_NONU, VAR_GATE_K, VAR_GATE_K_NONU)
+_KDIAG = (CONST_GATE_K_DIAG, VAR_GATE_K_DIAG, CONST_GATE_K_DIAG_NONU, VAR_GATE_K_DIAG_NONU)
+_KGATE = (CONST_GATE_K, VAR_GATE_K, CONST_GATE_K_NONU, VAR_GATE_K_NONU) + _KDIAG   # unfused barriers
+_VAR = (VAR_Q2, VAR_Q2_NONU, VAR_Q2_DIAG, VAR_Q1, VAR_Q1_NONU, VAR_GATE_K, VAR_GATE_K_NONU, VAR_GATE_K_DIAG,
+        VAR_GATE_K_DIAG_NONU)
 _NONU = (CONST_Q2_NONU, VAR_Q2_NONU, CONST_Q1_NONU, VAR_Q1_NONU)
 _DENS = (Q2_DENS, Q1_DENS, DIFF_Q2_DENS, DIFF_Q1_DENS, DENS_K, DIFF_DENS_K)
 _SWAP = np.array([0, 2, 1, 3])  # index 2 b_hi + b_lo with the two bits exchanged
@@ -216,6 +220,21 @@ class FusedCircuit(Circuit):
         self._kinds.append(kind)
         self._inner = None
 
+    def _add_gate_diag_k(self, positions, variable, non_unitary):
+        if any(p < 0 for p in positions):
+            raise OverflowError("can't convert negative int to unsigned")
+        if not 1 <= len(positions) <= 6:
+            raise ValueError("the number of gate qubits must be in 1..6.")
+        if any(p >= self.qubits_number for p in positions):
+            raise ValueError("pos is out of the bound.")
+        if len(set(positions)) != len(positions):
+            raise ValueError("positions must be different.")
+        kind = (VAR_GATE_K_DIAG if variable else CONST_GATE_K_DIAG) if not non_unitary else \
+            (VAR_GATE_K_DIAG_NONU if variable else CONST_GATE_K_DIAG_NONU)
+        self._program.append((kind, tuple(positions)))   # a barrier, executed unfused like the k-qubit gates
+        self._kinds.append(kind)
+        self._inner = None
+
     def __del__(self):
         pass
 
@@ -262,6 +281,8 @@ class FusedCircuit(Circuit):
             return 4 ** len(inst[1]) if k in (DENS_K, DIFF_DENS_K) else 4 if k in (Q1_DENS, DIFF_Q1_DENS) else 16
         def gate_len(inst):
             k = inst[0]
+            if k in _KDIAG:
+                return 2 ** len(inst[1])
             return 4 ** len(inst[1]) if k in _KGATE else 16 if k in (CONST_Q2, VAR_Q2, CONST_Q2_NONU, VAR_Q2_NONU) else 4
         ks, prog = self._kinds, self._program
         diff = (DIFF_Q1_DENS, DIFF_Q2_DENS, DIFF_DENS_K)
@@ -294,7 +315,9 @@ class FusedCircuit(Circuit):
                   Q2_DENS: "get_q2_dens_op", Q1_DENS: "get_q1_dens_op", DIFF_Q2_DENS: "get_q2_dens_op_with_grad",
                   DIFF_Q1_DENS: "get_q1_dens_op_with_grad", DENS_K: "get_dens_op", DIFF_DENS_K: "get_dens_op_with_grad",
                   CONST_GATE_K: "add_const_gate", VAR_GATE_K: "add_var_gate", CONST_GATE_K_NONU: "add_const_gate_nonu",
-                  VAR_GATE_K_NONU: "add_var_gate_nonu"}
+                  VAR_GATE_K_NONU: "add_var_gate_nonu", CONST_GATE_K_DIAG: "add_const_gate_diag",
+                  VAR_GATE_K_DIAG: "add_var_gate_diag", CONST_GATE_K_DIAG_NONU: "add_const_gate_diag_nonu",
+                  VAR_GATE_K_DIAG_NONU: "add_var_gate_diag_nonu"}
         self._xkinds = []
         for t, x in self._exec:
             if t == "kgate":

@@ -173,6 +173,11 @@ class AutoGradCircuit:
     def add_var_gate(self, positions): self.circuit.add_var_gate(positions)
     def add_const_gate_nonu(self, positions): self.circuit.add_const_gate_nonu(positions)
     def add_var_gate_nonu(self, positions): self.circuit.add_var_gate_nonu(positions)
+    # diagonal gates on 1..6 qubits, positions[0] the most significant bit (Circuit.add_const_gate_diag)
+    def add_const_gate_diag(self, positions): self.circuit.add_const_gate_diag(positions)
+    def add_var_gate_diag(self, positions): self.circuit.add_var_gate_diag(positions)
+    def add_const_gate_diag_nonu(self, positions): self.circuit.add_const_gate_diag_nonu(positions)
+    def add_var_gate_diag_nonu(self, positions): self.circuit.add_var_gate_diag_nonu(positions)
 
     def build(self) -> Tuple[Callable, Callable]:
         """Returns (simple_run, autodiff_run), src/qdc/circuit.py:160-202.

@@ -24,10 +24,12 @@ import numpy as np
 
 from .._ffi import Lib, ProfileEntry, QdcError, Stats, default_precision, get_lib
 
-# enum Instruction, src/circuit.rs:53-68, then the densities and the gates on 3..6 qubits (include/qdc_circuit.h)
+# enum Instruction, src/circuit.rs:53-68, then the densities and the gates on 3..6 qubits and the diagonal gates on
+# 1..6 qubits (include/qdc_circuit.h)
 (CONST_Q2, VAR_Q2, CONST_Q2_NONU, VAR_Q2_NONU, CONST_Q2_DIAG, VAR_Q2_DIAG, CONST_Q1, CONST_Q1_NONU, VAR_Q1,
  VAR_Q1_NONU, Q2_DENS, Q1_DENS, DIFF_Q2_DENS, DIFF_Q1_DENS, DENS_K, DIFF_DENS_K, CONST_GATE_K, VAR_GATE_K,
- CONST_GATE_K_NONU, VAR_GATE_K_NONU) = range(20)
+ CONST_GATE_K_NONU, VAR_GATE_K_NONU, CONST_GATE_K_DIAG, VAR_GATE_K_DIAG, CONST_GATE_K_DIAG_NONU,
+ VAR_GATE_K_DIAG_NONU) = range(24)
 
 (N_INSTRUCTIONS, N_CONST_GATES, N_VAR_GATES, N_DENSITIES, N_DIFF_DENSITIES, RUN_OUT_LEN, FORWARD_OUT_LEN,
  BACKWARD_OUT_LEN) = range(8)
@@ -41,7 +43,8 @@ class Circuit:
         self._lib.call("qdc_circuit_new", C.byref(h), self.qubits_number)
         self._h = h
         self._kinds: List[int] = []
-        self._dims: List[int] = []   # side of every instruction's density output or k-qubit gate matrix (else 0)
+        self._dims: List[int] = []   # side of every instruction's density output or k-qubit gate matrix, length of a
+                                     # diagonal k-qubit gate (else 0)
 
     def __del__(self):
         try:
@@ -85,6 +88,16 @@ class Circuit:
         self._lib.call("qdc_circuit_add_gate", self._h, pos.ctypes.data, pos.size, int(variable), int(non_unitary))
         self._kinds.append((VAR_GATE_K if variable else CONST_GATE_K) if not non_unitary
                            else (VAR_GATE_K_NONU if variable else CONST_GATE_K_NONU))
+        self._dims.append(1 << pos.size)
+
+    def _add_gate_diag_k(self, positions: List[int], variable: bool, non_unitary: bool):
+        if any(p < 0 for p in positions):
+            raise OverflowError("can't convert negative int to unsigned")
+        pos = np.array(positions, dtype=np.uintp)
+        self._lib.call("qdc_circuit_add_gate_diag", self._h, pos.ctypes.data, pos.size, int(variable),
+                       int(non_unitary))
+        self._kinds.append((VAR_GATE_K_DIAG if variable else CONST_GATE_K_DIAG) if not non_unitary
+                           else (VAR_GATE_K_DIAG_NONU if variable else CONST_GATE_K_DIAG_NONU))
         self._dims.append(1 << pos.size)
 
     def add_q2_const_gate(self, pos2: int, pos1: int): self._add(CONST_Q2, pos2, pos1)
@@ -140,6 +153,32 @@ class Circuit:
                 pos[0], pos[1])
         else:
             self._add_gate_k(pos, variable, non_unitary)
+
+    def add_const_gate_diag(self, positions: Sequence[int]):
+        """Diagonal gate on the qubits `positions` = [p_{k-1}, ..., p_0] (1 <= k <= 6, distinct, any order),
+        positions[0] the most significant bit of its index j: psi'[j, rest] = d[j] psi[j, rest].  d is taken flat
+        (2^k entries) from the constant gate list.  k = 2 is add_q2_const_gate_diag(p2, p1)."""
+        self._add_gate_diag(positions, False, False)
+
+    def add_var_gate_diag(self, positions: Sequence[int]):
+        """`add_const_gate_diag` from the variable gate list: backward returns its (2^k-entry) gradient
+        G[j] = sum_rest bwd[j, rest] fwd[j, rest]."""
+        self._add_gate_diag(positions, True, False)
+
+    def add_const_gate_diag_nonu(self, positions: Sequence[int]):
+        """`add_const_gate_diag` for a non-unitary d (the reverse pass un-computes with 1 / d)."""
+        self._add_gate_diag(positions, False, True)
+
+    def add_var_gate_diag_nonu(self, positions: Sequence[int]):
+        """`add_var_gate_diag` for a non-unitary d."""
+        self._add_gate_diag(positions, True, True)
+
+    def _add_gate_diag(self, positions, variable: bool, non_unitary: bool):
+        pos = [int(p) for p in positions]
+        if len(pos) == 2 and not non_unitary:
+            (self.add_q2_var_gate_diag if variable else self.add_q2_const_gate_diag)(pos[0], pos[1])
+        else:
+            self._add_gate_diag_k(pos, variable, non_unitary)
 
     def _add_dens(self, positions, with_grad: bool):
         pos = [int(p) for p in positions]
@@ -213,6 +252,8 @@ class Circuit:
                 res.append(out[o:o + 4].copy()); o += 4
             elif k in (VAR_GATE_K, VAR_GATE_K_NONU):
                 res.append(out[o:o + m * m].copy()); o += m * m
+            elif k in (VAR_GATE_K_DIAG, VAR_GATE_K_DIAG_NONU):
+                res.append(out[o:o + m].copy()); o += m
         assert o == n_out.value
         return res
 

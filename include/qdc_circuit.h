@@ -32,14 +32,16 @@ typedef struct qdc_circuit qdc_circuit;
 
 /* Instruction kinds == `enum Instruction`, src/circuit.rs:53-68 (same order),
  * then the densities on 3..6 qubits, which only qdc_circuit_add_dens adds,
- * then the gates on 3..6 qubits, which only qdc_circuit_add_gate adds. */
+ * then the gates on 3..6 qubits, which only qdc_circuit_add_gate adds,
+ * then the diagonal gates on 1..6 qubits, which only qdc_circuit_add_gate_diag adds. */
 enum qdc_kind {
   QDC_CONST_Q2 = 0, QDC_VAR_Q2 = 1, QDC_CONST_Q2_NONU = 2, QDC_VAR_Q2_NONU = 3,
   QDC_CONST_Q2_DIAG = 4, QDC_VAR_Q2_DIAG = 5,
   QDC_CONST_Q1 = 6, QDC_CONST_Q1_NONU = 7, QDC_VAR_Q1 = 8, QDC_VAR_Q1_NONU = 9,
   QDC_Q2_DENS = 10, QDC_Q1_DENS = 11, QDC_DIFF_Q2_DENS = 12, QDC_DIFF_Q1_DENS = 13,
   QDC_DENS_K = 14, QDC_DIFF_DENS_K = 15,
-  QDC_CONST_GATE_K = 16, QDC_VAR_GATE_K = 17, QDC_CONST_GATE_K_NONU = 18, QDC_VAR_GATE_K_NONU = 19
+  QDC_CONST_GATE_K = 16, QDC_VAR_GATE_K = 17, QDC_CONST_GATE_K_NONU = 18, QDC_VAR_GATE_K_NONU = 19,
+  QDC_CONST_GATE_K_DIAG = 20, QDC_VAR_GATE_K_DIAG = 21, QDC_CONST_GATE_K_DIAG_NONU = 22, QDC_VAR_GATE_K_DIAG_NONU = 23
 };
 
 /* qdc_circuit_count selectors */
@@ -76,7 +78,7 @@ const char* qdc_circuit_free(qdc_circuit* c);
 const char* qdc_circuit_set_state_from_host(qdc_circuit* c, const qdc_complex* host_state, size_t len);
 /* The 14 builder methods, src/circuit.rs:108-162.  pos1 is ignored for q1 kinds.
  * QDC_DENS_K / QDC_DIFF_DENS_K are refused here (they need qdc_circuit_add_dens), and so are
- * QDC_*_GATE_K* (they need qdc_circuit_add_gate). */
+ * QDC_*_GATE_K (they need qdc_circuit_add_gate) and QDC_*_GATE_K_DIAG* (qdc_circuit_add_gate_diag). */
 const char* qdc_circuit_add(qdc_circuit* c, int kind, size_t pos2, size_t pos1);
 /* Reduced density matrix on k = 1..6 distinct qubits positions[0..k-1] (positions[0] is the most
  * significant bit of the row and column index), with gradient if `with_grad`:
@@ -98,6 +100,19 @@ const char* qdc_circuit_add_dens(qdc_circuit* c, const size_t* positions, size_t
  * no instruction across it. */
 const char* qdc_circuit_add_gate(qdc_circuit* c, const size_t* positions, size_t k, int variable,
                                  int non_unitary);
+/* Diagonal gate on k = 1..6 distinct qubits positions[0..k-1] (positions[0] is the most significant bit
+ * of the index j), constant or `variable` (with gradient), unitary or `non_unitary`:
+ *   psi'[j, rest] = d[j] psi[j, rest],   d: 2^k entries, taken in program order from the const / var
+ *   gate lists like every other gate.
+ * The reverse pass un-computes with conj(d) (1 / d for non_unitary, in double precision; a zero entry
+ * fails with "U(j, j) is zero."), returns G[j] = sum_rest bwd[j, rest] fwd[j, rest] (2^k entries, no
+ * conjugation, like the two-qubit diagonal's gradient) and pulls the adjoint back with d (U^T = U).
+ * A variable gate after the last differentiable density has a zero gradient, like every gate kind.
+ * A unitary gate on k = 2 adds QDC_{CONST,VAR}_Q2_DIAG(positions[0], positions[1]); every other case
+ * adds QDC_{CONST,VAR}_GATE_K_DIAG[_NONU], a barrier like a density (the executor moves no instruction
+ * across it) that needs none of its qubits local on a sharded register: it costs no exchange. */
+const char* qdc_circuit_add_gate_diag(qdc_circuit* c, const size_t* positions, size_t k, int variable,
+                                      int non_unitary);
 size_t qdc_circuit_count(const qdc_circuit* c, int what);
 
 /* Circuit::run, src/circuit.rs:164-212 (all densities, program order). */
