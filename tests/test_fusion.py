@@ -162,7 +162,7 @@ def test_autograd_circuit_with_fusion_matches_the_plain_one():
 @pytest.mark.parametrize("seed", range(8))
 def test_random_programs_fuse_exactly(seed):
     """Random programs over every instruction kind: fused program + chain rule == original (oracle VM)."""
-    from test_scheduler import _random_program
+    from random_programs import _random_program
     rng = np.random.default_rng(200 + seed)
     n = 6
     o, const, var = _random_program(rng, n, 50)

@@ -12,6 +12,7 @@ import pytest
 from oracle import plan as op
 from oracle.circuit import OracleCircuit
 from conftest import haar_unitary
+from random_programs import _random_program, all_kinds_program, unitary_program
 from test_oracle import autodiff_gates, build_autodiff_circuit, tsallis_loss_and_cotangents
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -282,49 +283,16 @@ def test_sharded_execution_over_gloo(case, world, tile_bits):
     assert results[0][4] >= 1, "the sharded plan must contain at least one exchange"
 
 
-def _random_program(rng, n, length):
-    """A random program over all 14 instruction kinds (gates on random qubits, densities sprinkled in)."""
-    o = OracleCircuit(n)
-    const, var = [], []
-    adders2 = ("add_q2_const_gate", "add_q2_var_gate", "add_q2_const_gate_nonu", "add_q2_var_gate_nonu",
-               "add_q2_const_gate_diag", "add_q2_var_gate_diag")
-    adders1 = ("add_q1_const_gate", "add_q1_const_gate_nonu", "add_q1_var_gate", "add_q1_var_gate_nonu")
-    for _ in range(length):
-        r = rng.random()
-        if r < 0.55:
-            name = adders2[rng.integers(len(adders2))]
-            a, b = rng.choice(n, size=2, replace=False)
-            getattr(o, name)(int(a), int(b))
-            if name.endswith("diag"):
-                g = np.exp(1j * rng.normal(size=4))
-            else:
-                g = haar_unitary(rng, 4)
-                if name.endswith("nonu"):
-                    g = g + 0.05 * (rng.normal(size=16) + 1j * rng.normal(size=16))
-            (var if "_var_" in name else const).append(g)
-        elif r < 0.85:
-            name = adders1[rng.integers(len(adders1))]
-            getattr(o, name)(int(rng.integers(n)))
-            g = haar_unitary(rng, 2)
-            if name.endswith("nonu"):
-                g = g + 0.05 * (rng.normal(size=4) + 1j * rng.normal(size=4))
-            (var if "_var_" in name else const).append(g)
-        elif r < 0.93:
-            a, b = rng.choice(n, size=2, replace=False)
-            (o.get_q2_dens_op_with_grad if rng.random() < 0.7 else o.get_q2_dens_op)(int(a), int(b))
-        else:
-            (o.get_q1_dens_op_with_grad if rng.random() < 0.7 else o.get_q1_dens_op)(int(rng.integers(n)))
-    o.get_q2_dens_op_with_grad(1, 0)
-    return o, const, var
-
-
 @pytest.mark.parametrize("seed", range(8))
 def test_random_programs_are_scheduled_exactly(pkg, seed):
-    """Random programs over every instruction kind, every tiling strategy, single GPU and sharded: the plan
-    executed by the oracle's interpreter reproduces the program-order densities and gradients."""
+    """Random programs over every instruction kind, and programs of the two families of the GPU differential tests
+    (tests/random_programs.py), every tiling strategy, single GPU and sharded: the plan executed by the oracle's
+    interpreter reproduces the program-order densities and gradients."""
     rng = np.random.default_rng(100 + seed)
     n = 7
-    o, const, var = _random_program(rng, n, 40)
-    for strategy in (0, 1, 2):
-        for g, tile_bits in ((0, 5), (2, 4), (1, 0)):
-            check_plan(pkg, o, const, var, n, n - g, tile_bits, 2 if tile_bits else 0, tile_strategy=strategy)
+    programs = (_random_program(rng, n, 40), unitary_program(n, 300 + seed, 60),
+                all_kinds_program(n, 400 + seed, 60, k_rate=0))
+    for o, const, var in programs:
+        for strategy in (0, 1, 2):
+            for g, tile_bits in ((0, 5), (2, 4), (1, 0)):
+                check_plan(pkg, o, const, var, n, n - g, tile_bits, 2 if tile_bits else 0, tile_strategy=strategy)
